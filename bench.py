@@ -1,6 +1,6 @@
 """Benchmark of the JAMIE hot path on B200: train cells/sec (fwd + bwd + clip + Adam) of the coupled VAE.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 Workload (BASELINE.json configs[3], the configuration the metric is quoted on, at EVERY N): synthetic 1M-cell pair,
@@ -23,6 +23,8 @@ reference's random init (torch seed 666). A "step" is one optimizer step over on
   cpu_baseline  : the reference itself (oracle/_ref = a copy of /root/reference/jamie made by build()) timed on this
           box's host cores; falls back to the numpy oracle port when the copy is absent
 `--impl reference` times the reference alone (all host cores; rank 0 only under torchrun).
+`--dump-outputs DIR` writes what the last timed step left to its caller as DIR/<name>.npy (see dump_outputs); the inputs
+depend on the arguments only, so two builds can be compared output for output.
 """
 import argparse
 import contextlib
@@ -157,19 +159,20 @@ def cpu_reference(steps, warmup, n=4096):
         JJ.time_logger = base
     hist = max((lg.history for lg in loggers), key=lambda h: len(h.get('Step', [])))
     labels = [k for k in hist if k not in ('Setup', 'Output')]
-    avail = len(hist['Step'])
-    w = min(warmup, max(0, avail - steps))
-    k = min(steps, avail - w)
+    w, k = warmup, steps
+    if len(hist['Step']) < w + k:
+        raise RuntimeError(f'the reference ran {len(hist["Step"])} optimizer steps, {w + k} were asked for')
     total = sum(float(np.sum(hist[lb][w:w + k])) for lb in labels if len(hist[lb]) >= w + k)
     return {'value': BATCH * k / total, 'unit': 'cells/s', 'cores': os.cpu_count(), 'kind': 'reference',
-            'threads': torch.get_num_threads(), 'ms_per_step': 1e3 * total / k,
+            'threads': torch.get_num_threads(), 'ms_per_step': 1e3 * total / k, 'steps': k, 'warmup': w,
             'sample': f'{k} optimizer steps (after {w} warm-up) of the reference\'s own project_jamie loop, batch {BATCH}, widths '
                       f'{DIMS}, output_dim {LATENT}, dropout {DROPOUT}, n = {n} cells, torch {torch.__version__} CPU; sum of '
                       f'its time_logger laps {labels}, {total:.1f} s'}
 
 
-def cpu_port(seconds=12.0, max_steps=200):
-    """Fallback when the reference copy is absent: the numpy oracle port of one reference optimizer step."""
+def cpu_port(steps, warmup):
+    """Fallback when the reference copy is absent: the numpy oracle port of one reference optimizer step, timed over
+    `steps` steps after `warmup`."""
     from oracle import jamie_oracle as O
     rng = np.random.default_rng(0)
     n = 8192
@@ -193,17 +196,16 @@ def cpu_port(seconds=12.0, max_steps=200):
         masks = [(rng.random((BATCH, w)) >= DROPOUT).astype(np.uint8) for w in widths]
         orc.train_step(x, corr, np.zeros((BATCH, BATCH), np.float32), eps, masks, 0.5)
 
-    for s in range(2):
+    for s in range(warmup):
         one(s)
     t0 = time.perf_counter()
-    steps = 0
-    while steps < max_steps and time.perf_counter() - t0 < seconds:
-        one(steps)
-        steps += 1
+    for s in range(steps):
+        one(s)
     dt = time.perf_counter() - t0
     return {'value': BATCH * steps / dt, 'unit': 'cells/s', 'cores': os.cpu_count(), 'kind': 'port',
-            'sample': f'{steps} optimizer steps of batch {BATCH} at widths {DIMS}, output_dim {LATENT} '
-                      f'(numpy fp32 oracle, BLAS on all host cores), {dt:.1f} s', 'ms_per_step': 1e3 * dt / steps}
+            'sample': f'{steps} optimizer steps (after {warmup} warm-up) of batch {BATCH} at widths {DIMS}, output_dim {LATENT} '
+                      f'(numpy fp32 oracle, BLAS on all host cores), {dt:.1f} s', 'ms_per_step': 1e3 * dt / steps,
+            'steps': steps, 'warmup': warmup}
 
 
 def cpu_baseline(steps=60, warmup=10):
@@ -212,21 +214,20 @@ def cpu_baseline(steps=60, warmup=10):
         try:
             return cpu_reference(steps, warmup)
         except Exception as ex:   # a broken copy must not take the GPU numbers down with it
-            cb = cpu_port()
+            cb = cpu_port(steps, warmup)
             cb['note'] = f'reference copy failed to run ({type(ex).__name__}: {ex}); oracle port timed instead'
             return cb
-    return cpu_port()
+    return cpu_port(steps, warmup)
 
 
 def run_reference(args):
     rank = int(os.environ.get('RANK', 0))
     if rank != 0:
         return
-    steps = max(3, min(args.steps, 200))
-    cb = cpu_baseline(steps=steps, warmup=max(3, min(args.warmup, 20)))
+    cb = cpu_baseline(steps=args.steps, warmup=args.warmup)
     line = {
         'impl': 'reference', 'metric': 'train cells/sec (fwd+bwd+Adam)', 'value': cb['value'], 'unit': 'cells/s',
-        'n_gpus': args.gpus, 'steps': args.steps, 'warmup': args.warmup, 'ms_per_step': cb['ms_per_step'],
+        'n_gpus': args.gpus, 'steps': cb['steps'], 'warmup': cb['warmup'], 'ms_per_step': cb['ms_per_step'],
         'higher_is_better': True, 'scaling': 'weak', 'vs_baseline': None, 'dtype': 'f32', 'data': 'synthetic',
         'config': workload_config(args.gpus),
         'cpu_baseline': cb,
@@ -312,6 +313,22 @@ def fit_transform_leg(torch, n=100_000, epochs=10):
                     'training, final encode, download; marginal_us_per_step = (T(10 epochs) - T(1 epoch)) / extra steps'}
 
 
+def dump_outputs(eng, last_losses, out_dir):
+    """The results of the last timed optimizer step, float32, packed in the reference's parameter / BatchNorm order:
+    losses (KL, Rec, CosSim, F, total, pre-clip gradient norm), grads (that step's gradients), params and bn_stats
+    (running mean, running var per BatchNorm layer) after its update. 34.5 MB at the benchmark's shape."""
+    os.makedirs(out_dir, exist_ok=True)
+    bn = eng.get_bn_stats()
+    arrays = {
+        'losses': np.asarray(last_losses[:6], np.float32),
+        'grads': np.concatenate([g.ravel() for g in eng.get_grads()]),
+        'params': eng.get_params(as_list=False),
+        'bn_stats': np.concatenate([v for k, v in bn.items() if not k.endswith('.num_batches_tracked')]),
+    }
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), a)
+
+
 def workload_config(n_gpus):
     wl = f'BASELINE configs[3]: synthetic 1M-cell pair sharded over {n_gpus} rank(s), widths [512,512], output_dim 32, ' \
          f'batch 512 per rank, 50% partially matched diagonal P (hybrid sampler), dropout 0.6, F=0' + \
@@ -332,7 +349,12 @@ def main():
     ap.add_argument('--no-fit', action='store_true')
     ap.add_argument('--predict-only', action='store_true', help='modal_predict leg alone (tuning runs)')
     ap.add_argument('--profile', action='store_true', help='device-resident steps only (for ncu): no e2e / stage / CPU legs, no JSON line')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the results of the last timed step as DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be at least 1 and --warmup at least 0')
+    if args.dump_outputs and (args.impl == 'reference' or args.predict_only):
+        ap.error('--dump-outputs writes the results of the timed training steps: not with --impl reference or --predict-only')
     if args.impl == 'reference':
         return run_reference(args)
 
@@ -434,6 +456,8 @@ def main():
     assert finite_rows[-max(1, (W + K) // 10):].all() and nonfinite_steps <= max(1, (W + K) // 100), \
         f'non-finite losses in the timed region: {nonfinite_steps} of {W + K} steps'
     value = BATCH * K * world / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:     # before the legs below train the same engine further
+        dump_outputs(eng, losses[-1], args.dump_outputs)
 
     if args.profile:
         print(f'profile run: {ms / K * 1e3:.1f} us/step', flush=True)

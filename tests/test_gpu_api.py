@@ -48,6 +48,7 @@ def test_fit_transform_end_to_end(capsys):
     pred1 = jm.modal_predict(data[0], 0)
     assert pred1.shape == data[1].shape and pred1.dtype == np.float64
     assert np.nanmean(imputation_correlation(pred1, data[1])) > 0.7
+    jm.engine.close()
 
 
 def test_ingest_pca_projection_runs_on_the_engine():
@@ -97,6 +98,8 @@ def test_save_load_roundtrip(tmp_path):
     keys = list(jm2.model.state_dict().keys())
     assert keys[0] == 'sigma' and 'encoders.0.0.weight' in keys and 'decoders.1.8.bias' in keys
     assert 'encoders.0.1.running_mean' in keys and len(keys) == 45 + 24
+    jm.engine.close()
+    jm2.engine.close()
 
 
 def test_load_reference_checkpoint():
@@ -109,6 +112,7 @@ def test_load_reference_checkpoint():
         got = jm.modal_predict(io[f'data{i}'], i)
         assert U.rel(got, io[f'pred{i}']) < 3e-3
         assert U.rel(jm.transform_one(io[f'data{i}'], i), io[f'tone{i}']) < 3e-3
+    jm.engine.close()
 
 
 def test_early_stop_fires_at_the_epoch_the_reference_rule_gives():
@@ -122,6 +126,7 @@ def test_early_stop_fires_at_the_epoch_the_reference_rule_gives():
     jm = JAMIE(output_dim=8, batch_size=128, pca_dim=None, use_f_tilde=False, log_DNN=10 ** 6, **kw)
     jm.fit_transform(dataset=data)
     ran = len(jm.loss_history['KL'])
+    jm.engine.close()
     assert jm.epochs_run == ran
     total = np.sum([np.asarray(jm.loss_history[k], np.float64) for k in ('KL', 'Rec', 'CosSim', 'F')], axis=0)
     best, streak, want = np.inf, 0, kw['epoch_DNN']

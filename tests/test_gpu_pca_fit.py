@@ -77,6 +77,7 @@ def test_fit_transform_uses_the_gpu_pca_fit_and_matches_the_host_fit():
                    pca_fit=how)
         jm.fit_transform(dataset=[d.copy() for d in data])
         pres[how] = [np.asarray(jm.dataset[i]) for i in range(2)], [jm.model.preprocessing[i].__self__.pca for i in range(2)]
+        jm.engine.close()
     from sklearn.decomposition import PCA
     for i in range(2):
         assert isinstance(pres['gpu'][1][i], PCA)
@@ -100,6 +101,7 @@ def test_sparse_input_matches_dense_through_the_api():
         jm = JAMIE(output_dim=8, batch_size=64, pca_dim=[20, 16], epoch_DNN=3, min_epochs=1, use_f_tilde=False, manual_seed=5)
         emb = jm.fit_transform(dataset=[(sp.csr_matrix(d) if how == 'sparse' else d.copy()) for d in data])
         outs[how] = [np.asarray(jm.dataset[i]) for i in range(2)], emb, jm.modal_predict(sp.csr_matrix(data[0]) if how == 'sparse' else data[0], 0)
+        jm.engine.close()
     for i in range(2):
         np.testing.assert_allclose(outs['sparse'][0][i], outs['dense'][0][i], atol=1e-5)
         np.testing.assert_allclose(outs['sparse'][1][i], outs['dense'][1][i], atol=1e-4)

@@ -8,6 +8,17 @@ from oracle import jamie_oracle as O
 from tests.golden_util import CASES, Golden
 
 
+@pytest.fixture(autouse=True)
+def host_projection():
+    """These tests pin the host arithmetic. In a session that also ran GPU tests, the engine of a JAMIE model that was
+    never closed stays attached as the process's PCA projector and would take preclass onto the GPU (fp32 class)."""
+    from jamie_b200 import utilities as Ut
+    attached = Ut._GPU_PROJECTOR
+    Ut.set_gpu_projector(None)
+    yield
+    Ut.set_gpu_projector(attached)
+
+
 @pytest.mark.parametrize('name', ['diag_drop', 'rep_F', 'zeros_unequal'])
 def test_initial_weights_equal_reference(name):
     """Same torch seed + same construction order => bit-identical initial parameters as the reference model."""
@@ -196,6 +207,7 @@ def test_bench_reference_arm_prints_one_json_line():
     assert len(lines) == 1
     d = json.loads(lines[0])
     assert d['impl'] == 'reference' and d['unit'] == 'cells/s' and d['higher_is_better'] is True and d['value'] > 0
+    assert (d['steps'], d['warmup']) == (2, 3) and (d['cpu_baseline']['steps'], d['cpu_baseline']['warmup']) == (2, 3)
     assert d['cpu_baseline']['kind'] in ('reference', 'port') and d['cpu_baseline']['cores'] >= 1
     assert d['e2e'] == {'value': d['value'], 'unit': 'cells/s', 'h2d_bytes_per_step': 0, 'd2h_bytes_per_step': 0}
     assert d['config']['workload'].startswith('BASELINE configs[3]')
