@@ -212,6 +212,33 @@ int jb_metric_knn_vote(const float* query, long long nq, const float* ref, const
                        int k, int n_classes, int device, int* pred_class);
 int jb_metric_feature_pearson(const float* x, const float* y, long long n, long long d, int device, double* r);
 
+/* Distances of the F estimation (compute_distances, jamie/jamie.py:839-890; the default distance_mode 'geodesic' is
+ * unioncom.utils.geodesic_distances of unioncom==0.4.0, restated and unpinned in jamie_b200/correspondence.py).
+ * A jb_dist handle owns one n x n float64 matrix D on one device and a stream; host pointers throughout.
+ *   jb_dist_create    : D = 0. Fails with a message when the 8 n^2 bytes of D do not fit in the device's free memory.
+ *   jb_dist_accumulate: D[i, j] += sum_c f(slab[i, c], slab[j, c]) over a [n, w] float64 host slab with row pitch ld;
+ *                       kind 0 = (a - b)^2, 1 = |a - b|, 2 = a b (the caller streams the columns of the data in slabs,
+ *                       after row normalising / centring / ranking for the product forms). Columns are summed in order
+ *                       (any slab widths give the same bits); D stays bitwise symmetric, diagonal exactly 0 for kinds 0
+ *                       and 1. Asynchronous; `slab` may be reused when the call returns.
+ *   jb_dist_finish    : transform 0 = none, 1 = sqrt (euclidean), 2 = 1 - g clipped to [0, 2] with a zero diagonal
+ *                       (sklearn cosine_distances, scipy correlation), 3 = (1 - clip(g, -1, 1)) / 2 (np.corrcoef /
+ *                       spearmanr for 'pearson' / 'spearman', jamie/jamie.py:851-884); NaN stays NaN. out [n, n] or NULL.
+ *   jb_dist_knn       : per row the k nearest columns of D in ascending order, equal distances by the lowest column (a
+ *                       stable argsort; the row itself counts, as in kneighbors_graph(X)). idx [n, k], dist [n, k] or
+ *                       NULL. The lists stay on the device for jb_dist_geodesic. D must be non-negative.
+ *   jb_dist_geodesic  : all-pairs shortest paths on the undirected graph of the first k (<= the jb_dist_knn k) neighbours
+ *                       (blocked Floyd-Warshall in float64, overwriting D), then every pair above the largest finite
+ *                       distance set to twice that distance. out [n, n] or NULL.
+ * All but jb_dist_accumulate synchronise the handle's stream before they return. */
+typedef struct jb_dist jb_dist;
+int jb_dist_create(long long n, int device, jb_dist** out);
+void jb_dist_destroy(jb_dist* h);
+int jb_dist_accumulate(jb_dist* h, int kind, const double* slab, long long w, long long ld);
+int jb_dist_finish(jb_dist* h, int transform, double* out);
+int jb_dist_knn(jb_dist* h, int k, int* idx, double* dist);
+int jb_dist_geodesic(jb_dist* h, int k, double* out);
+
 /* Debug / parity taps: copy a named intermediate of the last step to the host (synchronises).
  * Names: "x0","y1_0","h1_0","y2_0","h2_0","mulv0","z0","c0","xhat0", ... (see csrc/engine.cu: tap table),
  * "corr", "fblk", "grad" (padded flat), "theta". Returns the number of floats written, or -1. */

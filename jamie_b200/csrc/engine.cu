@@ -33,6 +33,7 @@
 #include "hgemm.cuh"
 #include "stepk.cuh"
 #include "metrics.cuh"
+#include "distances.cuh"
 
 namespace {
 
@@ -819,6 +820,19 @@ int metric_grid(long long tiles) {
   return static_cast<int>(tiles < g ? (tiles > 0 ? tiles : 1) : g);
 }
 }  // namespace
+
+struct jb_dist {   // one n x n float64 distance matrix on one device (jb_dist_*)
+  long long n = 0;
+  int device = 0;
+  cudaStream_t s = nullptr;
+  double* D = nullptr;
+  double* slab = nullptr;   // device copy of the current column slab
+  size_t slab_cap = 0;      // doubles
+  int* knn_idx = nullptr;   // [n, knn_k] neighbour lists of the last jb_dist_knn
+  double* knn_dist = nullptr;
+  int knn_k = 0;
+  unsigned long long* scratch = nullptr;
+};
 
 extern "C" {
 
@@ -1738,6 +1752,131 @@ int jb_metric_feature_pearson(const float* x, const float* y, long long n, long 
     const double cxy = m[4] - m[0] * m[1] / N, cxx = m[2] - m[0] * m[0] / N, cyy = m[3] - m[1] * m[1] / N;
     r[c] = cxy / std::sqrt(cxx * cyy);   // constant feature: 0 / 0 = nan, as the host definition gives
   }
+  return 0;
+}
+
+// ---------------------------------------------------------------------------------------------- F-estimation distances (N2)
+
+int jb_dist_create(long long n, int device, jb_dist** out) {
+  if (!out) return fail("null argument");
+  *out = nullptr;
+  if (n < 1 || n > (1LL << 31) - 1) return fail("bad number of rows %lld", n);
+  CU(cudaSetDevice(device));
+  size_t free_b = 0, total_b = 0;
+  CU(cudaMemGetInfo(&free_b, &total_b));
+  const double need = 8.0 * static_cast<double>(n) * static_cast<double>(n);
+  if (need > static_cast<double>(free_b))
+    return fail("n = %lld rows need %.2f GB for the n x n float64 distance matrix; %.2f GB of device %d are free", n, need / 1e9,
+                free_b / 1e9, device);
+  jb_dist* h = new jb_dist();
+  h->n = n;
+  h->device = device;
+  cudaError_t ce = cudaStreamCreateWithFlags(&h->s, cudaStreamNonBlocking);
+  if (ce == cudaSuccess) ce = cudaMalloc(&h->D, static_cast<size_t>(n) * n * sizeof(double));
+  if (ce == cudaSuccess) ce = cudaMalloc(&h->scratch, sizeof(unsigned long long));
+  if (ce == cudaSuccess) ce = cudaMemsetAsync(h->D, 0, static_cast<size_t>(n) * n * sizeof(double), h->s);
+  if (ce != cudaSuccess) {
+    jb_dist_destroy(h);
+    return fail("distance handle of %lld rows: %s", n, cudaGetErrorString(ce));
+  }
+  *out = h;
+  return 0;
+}
+
+void jb_dist_destroy(jb_dist* h) {
+  if (!h) return;
+  cudaSetDevice(h->device);
+  if (h->s) cudaStreamSynchronize(h->s);
+  cudaFree(h->D); cudaFree(h->slab); cudaFree(h->knn_idx); cudaFree(h->knn_dist); cudaFree(h->scratch);
+  if (h->s) cudaStreamDestroy(h->s);
+  delete h;
+}
+
+int jb_dist_accumulate(jb_dist* h, int kind, const double* slab, long long w, long long ld) {
+  if (!h || !slab) return fail("null argument");
+  if (kind < jb::DIST_SQDIFF || kind > jb::DIST_PRODUCT) return fail("unknown distance kind %d", kind);
+  if (w < 1 || w > (1LL << 30) || ld < w) return fail("bad slab shape: %lld columns, row pitch %lld", w, ld);
+  CU(cudaSetDevice(h->device));
+  const size_t span = static_cast<size_t>(h->n - 1) * ld + w;
+  if (span > h->slab_cap) {
+    CU(cudaStreamSynchronize(h->s));
+    cudaFree(h->slab);
+    h->slab = nullptr; h->slab_cap = 0;
+    CU(cudaMalloc(&h->slab, span * sizeof(double)));
+    h->slab_cap = span;
+  }
+  // stream-ordered after the previous slab's kernel; from pageable memory it returns once `slab` has been staged
+  CU(cudaMemcpyAsync(h->slab, slab, span * sizeof(double), cudaMemcpyHostToDevice, h->s));
+  const long long tiles = (h->n + jb::DA_TILE - 1) / jb::DA_TILE;
+  const int grid = metric_grid(tiles * (tiles + 1) / 2);
+  const int wi = static_cast<int>(w);
+  if (kind == jb::DIST_SQDIFF) jb::k_dist_accum<jb::DIST_SQDIFF><<<grid, jb::DA_THREADS, 0, h->s>>>(h->slab, h->n, wi, ld, h->D);
+  else if (kind == jb::DIST_ABSDIFF) jb::k_dist_accum<jb::DIST_ABSDIFF><<<grid, jb::DA_THREADS, 0, h->s>>>(h->slab, h->n, wi, ld, h->D);
+  else jb::k_dist_accum<jb::DIST_PRODUCT><<<grid, jb::DA_THREADS, 0, h->s>>>(h->slab, h->n, wi, ld, h->D);
+  CU(cudaGetLastError());
+  return 0;
+}
+
+int jb_dist_finish(jb_dist* h, int transform, double* out) {
+  if (!h) return fail("null argument");
+  if (transform < jb::DIST_NONE || transform > jb::DIST_HALF_ONE_MINUS) return fail("unknown distance transform %d", transform);
+  CU(cudaSetDevice(h->device));
+  const size_t nn = static_cast<size_t>(h->n) * h->n;
+  if (transform != jb::DIST_NONE) {
+    jb::k_dist_finish<<<metric_grid(static_cast<long long>((nn + 255) / 256)), 256, 0, h->s>>>(h->D, h->n, transform);
+    CU(cudaGetLastError());
+  }
+  if (out) CU(cudaMemcpyAsync(out, h->D, nn * sizeof(double), cudaMemcpyDeviceToHost, h->s));
+  CU(cudaStreamSynchronize(h->s));
+  return 0;
+}
+
+int jb_dist_knn(jb_dist* h, int k, int* idx, double* dist) {
+  if (!h || !idx) return fail("null argument");
+  if (k < 1 || k > h->n || k > 16384) return fail("k = %d neighbours of %lld rows (1 .. min(n, 16384))", k, h->n);
+  CU(cudaSetDevice(h->device));
+  CU(cudaStreamSynchronize(h->s));
+  cudaFree(h->knn_idx); cudaFree(h->knn_dist);
+  h->knn_idx = nullptr; h->knn_dist = nullptr; h->knn_k = 0;
+  const size_t nk = static_cast<size_t>(h->n) * k;
+  CU(cudaMalloc(&h->knn_idx, nk * sizeof(int)));
+  CU(cudaMalloc(&h->knn_dist, nk * sizeof(double)));
+  const size_t smem = static_cast<size_t>(k) * (sizeof(unsigned long long) + sizeof(int));
+  CU(cudaFuncSetAttribute(jb::k_knn_rows, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+  jb::k_knn_rows<<<static_cast<unsigned>(h->n), jb::KN_THREADS, smem, h->s>>>(h->D, h->n, k, h->knn_idx, h->knn_dist);
+  CU(cudaGetLastError());
+  h->knn_k = k;
+  CU(cudaMemcpyAsync(idx, h->knn_idx, nk * sizeof(int), cudaMemcpyDeviceToHost, h->s));
+  if (dist) CU(cudaMemcpyAsync(dist, h->knn_dist, nk * sizeof(double), cudaMemcpyDeviceToHost, h->s));
+  CU(cudaStreamSynchronize(h->s));
+  return 0;
+}
+
+int jb_dist_geodesic(jb_dist* h, int k, double* out) {
+  if (!h) return fail("null argument");
+  if (h->knn_k < 1) return fail("jb_dist_geodesic needs the neighbour lists of jb_dist_knn first");
+  if (k < 1 || k > h->knn_k) return fail("k = %d, but the neighbour lists hold %d per row", k, h->knn_k);
+  CU(cudaSetDevice(h->device));
+  const long long n = h->n;
+  const size_t nn = static_cast<size_t>(n) * n;
+  const int eg = metric_grid(static_cast<long long>((nn + 255) / 256));
+  jb::k_graph_fill<<<eg, 256, 0, h->s>>>(h->D, n);
+  jb::k_graph_edges<<<static_cast<unsigned>((n * k + 255) / 256), 256, 0, h->s>>>(h->D, n, h->knn_idx, h->knn_dist, h->knn_k, k);
+  const int nb = static_cast<int>((n + jb::FW_B - 1) / jb::FW_B);
+  CU(cudaFuncSetAttribute(jb::k_fw_cross, cudaFuncAttributeMaxDynamicSharedMemorySize, jb::FW_CROSS_SMEM));
+  for (int kb = 0; kb < nb; ++kb) {
+    jb::k_fw_diag<<<1, jb::FW_THREADS, 0, h->s>>>(h->D, n, kb);
+    if (nb > 1) {
+      jb::k_fw_cross<<<dim3(nb - 1, 2), jb::FW_THREADS, jb::FW_CROSS_SMEM, h->s>>>(h->D, n, kb);
+      jb::k_fw_rest<<<dim3(nb, nb), jb::FW_THREADS, 0, h->s>>>(h->D, n, kb);
+    }
+  }
+  CU(cudaMemsetAsync(h->scratch, 0, sizeof(unsigned long long), h->s));
+  jb::k_finite_max<<<eg, 256, 0, h->s>>>(h->D, static_cast<long long>(nn), h->scratch);
+  jb::k_fill_unreachable<<<eg, 256, 0, h->s>>>(h->D, static_cast<long long>(nn), h->scratch);
+  CU(cudaGetLastError());
+  if (out) CU(cudaMemcpyAsync(out, h->D, nn * sizeof(double), cudaMemcpyDeviceToHost, h->s));
+  CU(cudaStreamSynchronize(h->s));
   return 0;
 }
 

@@ -8,7 +8,8 @@ numpy batch sampler (same draws, same order as the reference, so a seeded run vi
 bookkeeping, early stopping and printing.
 
 F estimation (``compute_distances`` + ``Prime_Dual``, jamie/jamie.py:224-414, 839-890) lives in ``correspondence.py``: the
-distances on the host with the reference's own sklearn / scipy calls, the primal-dual iteration on the GPU.  Out of scope:
+distances on the host with the reference's own sklearn / scipy calls (``distances='gpu'``: on the GPU, csrc/distances.cuh),
+the primal-dual iteration on the GPU.  Out of scope:
 the tsne projection branch, ``corr_method='jamie'`` (marked WIP in the reference), ``model_pca='umap'``.
 """
 import os
@@ -195,7 +196,8 @@ class JAMIE(UnionCom):
                  in_place=False, loss_weights=None, model_pca='pca', model_class=edModelVar, model_lr=1e-3,
                  dropout=None, pca_dim=2 * [512], batch_step=True, use_f_tilde=True, use_early_stop=True,
                  min_epochs=2500, min_increment=1e-8, max_steps_without_increment=500, debug=False, log_debug=100,
-                 record_loss=True, enable_memory_logging=False, device='cpu', sampler='auto', pca_fit='gpu', **kwargs):
+                 record_loss=True, enable_memory_logging=False, device='cpu', sampler='auto', pca_fit='gpu', distances='host',
+                 **kwargs):
         # sampler (not in the reference): 'reference' = the reference's numpy draws call for call; 'fast' = the same
         # distribution from an O(batch) draw; 'auto' = 'reference' up to FAST_SAMPLER_ROWS cells, 'fast' above.
         assert sampler in ('auto', 'reference', 'fast'), f"sampler must be 'auto', 'reference' or 'fast', not {sampler!r}"
@@ -204,6 +206,11 @@ class JAMIE(UnionCom):
         # covariance_eigh algorithm, exact PCA); 'sklearn' = the reference's host call PCA(n_components).fit_transform(data).
         assert pca_fit in ('gpu', 'sklearn'), f"pca_fit must be 'gpu' or 'sklearn', not {pca_fit!r}"
         self.pca_fit = pca_fit
+        # distances (not in the reference): 'host' = compute_distances with the reference's sklearn / scipy calls; 'gpu' = the
+        # same distances from the jb_dist kernels on the engine's device (correspondence.gpu_distance_function; a scipy.sparse
+        # modality is streamed in column slabs, never densified whole).
+        assert distances in ('host', 'gpu'), f"distances must be 'host' or 'gpu', not {distances!r}"
+        self.distances = distances
         self.match_result = match_result
         self.PF_Ratio = PF_Ratio
         self.corr_method = corr_method
@@ -316,16 +323,19 @@ class JAMIE(UnionCom):
     # ------------------------------------------------------------------------------------------------ F estimation
     def compute_distances(self, save_dist=True):
         """Helper function to compute distances for each dataset (jamie/jamie.py:839-890)"""
-        from .correspondence import distance_function
+        from .correspondence import distance_function, gpu_distance_function
         if save_dist:
             self.dist = []
+        gpu_fn = None
+        if save_dist and self.distances == 'gpu':
+            gpu_fn = gpu_distance_function(self.distance_mode, self.kmax, device=self._cuda_index())
         print('Shape of Raw data')
         for i in range(self.dataset_num):
             print('Dataset {}:'.format(i), np.shape(self.dataset[i]))
-            self.distance_function = distance_function(self.distance_mode, self.kmax)
+            self.distance_function = gpu_fn or distance_function(self.distance_mode, self.kmax)
             if save_dist:
                 data_i = self.dataset[i]
-                if hasattr(data_i, 'toarray') and not isinstance(data_i, np.ndarray):   # scipy.sparse (AnnData.X)
+                if gpu_fn is None and hasattr(data_i, 'toarray') and not isinstance(data_i, np.ndarray):   # scipy.sparse (AnnData.X)
                     data_i = data_i.toarray()
                 self.dist.append(self.distance_function(data_i))
 
