@@ -239,6 +239,34 @@ int jb_dist_finish(jb_dist* h, int transform, double* out);
 int jb_dist_knn(jb_dist* h, int k, int* idx, double* dist);
 int jb_dist_geodesic(jb_dist* h, int k, double* out);
 
+/* Randomized PCA fit (sklearn's randomized solver, jamie_b200/pca_fit.py randomized_fit_transform): a jb_pcaop handle
+ * holds one input matrix X [n, d] on one device and applies the implicitly centred Xc = X - 1 mu^T to thin dense
+ * matrices, so that no d x d matrix is ever formed. It owns a stream; host data are copied with cudaMemcpyAsync on it.
+ *   jb_pcaop_create_dense : dense fp32 rows [n, d] (host). Products: 3xTF32 split GEMM on hi/lo planes of Xc (the mean is
+ *                           subtracted during the split), long reductions chunked and accumulated in float64.
+ *   jb_pcaop_create_sparse: CSR of X and CSR of X^T (= CSC of X), host arrays: int64 indptr, int32 indices, fp32 values.
+ *                           Products: one CSR x dense kernel for both directions, each output summing its row's nonzeros
+ *                           in index order (fp32 values, float64 products and sums; long rows in fixed-size segments
+ *                           added in order), then the centring as a float64 rank-1 correction before the one rounding to
+ *                           fp32. No floating-point atomics: results are bit-reproducible.
+ *   Both refuse, with a message and before any allocation, inconsistent CSR input and an operand (plus its workspaces)
+ *   that does not fit in the device's free memory. mu = 0 until jb_pcaop_stats.
+ *   jb_pcaop_stats  : per-column mean and variance (ddof 0), float64, two passes (sum, then centred squares; for sparse
+ *                     input the (n - nnz_c) mu^2 of the zeros is added). mean [d], var [d] host or NULL. Stores mu in the
+ *                     handle for the centring. Synchronous.
+ *   jb_pcaop_apply  : trans 0: Y[n, l] = Xc B, with B [d, l].  trans 1: Y[d, l] = Xc^T B, with B [n, l].
+ *                     Packed row-major fp32 DEVICE pointers, asynchronous on `stream` (ordered after the work already on
+ *                     it; NULL = the legacy default stream). Workspaces for width l are allocated on first use; a width
+ *                     whose workspaces do not fit is refused like an operand that does not fit. */
+typedef struct jb_pcaop jb_pcaop;
+int jb_pcaop_create_dense(const float* X, long long n, long long d, int device, jb_pcaop** out);
+int jb_pcaop_create_sparse(long long n, long long d, long long nnz, const long long* row_ptr, const int* col_idx,
+                           const float* row_val, const long long* col_ptr, const int* row_idx, const float* col_val,
+                           int device, jb_pcaop** out);
+int jb_pcaop_stats(jb_pcaop* h, double* mean, double* var);
+int jb_pcaop_apply(jb_pcaop* h, int trans, const float* B, int l, float* Y, void* stream);
+void jb_pcaop_destroy(jb_pcaop* h);
+
 /* Debug / parity taps: copy a named intermediate of the last step to the host (synchronises).
  * Names: "x0","y1_0","h1_0","y2_0","h2_0","mulv0","z0","c0","xhat0", ... (see csrc/engine.cu: tap table),
  * "corr", "fblk", "grad" (padded flat), "theta". Returns the number of floats written, or -1. */

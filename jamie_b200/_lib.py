@@ -74,6 +74,11 @@ SIGNATURES = {
     'jb_dist_finish': (C.c_int, [_P, C.c_int, _P]),
     'jb_dist_knn': (C.c_int, [_P, C.c_int, _P, _P]),
     'jb_dist_geodesic': (C.c_int, [_P, C.c_int, _P]),
+    'jb_pcaop_create_dense': (C.c_int, [_P, _LL, _LL, C.c_int, C.POINTER(_P)]),
+    'jb_pcaop_create_sparse': (C.c_int, [_LL, _LL, _LL, _P, _P, _P, _P, _P, _P, C.c_int, C.POINTER(_P)]),
+    'jb_pcaop_stats': (C.c_int, [_P, _P, _P]),
+    'jb_pcaop_apply': (C.c_int, [_P, C.c_int, _P, C.c_int, _P, _P]),
+    'jb_pcaop_destroy': (None, [_P]),
     'jb_train_step_hostbatch': (C.c_int, [_P, _P, _P, _P, _P, C.c_int, C.c_double, _P, _P]),
     'jb_step_backward_hostbatch': (C.c_int, [_P, _P, _P, _P, _P, C.c_int, C.c_double, _P]),
     'jb_hostbatch_submit': (C.c_int, [_P, _P, _P, _P, _P, C.c_int, C.c_double, _P]),

@@ -34,6 +34,7 @@
 #include "stepk.cuh"
 #include "metrics.cuh"
 #include "distances.cuh"
+#include "pcaop.cuh"
 
 namespace {
 
@@ -820,6 +821,40 @@ int metric_grid(long long tiles) {
   return static_cast<int>(tiles < g ? (tiles > 0 ? tiles : 1) : g);
 }
 }  // namespace
+
+struct jb_pcaop {   // one centred PCA operand Xc = X - 1 mu^T on one device (jb_pcaop_*)
+  long long n = 0, d = 0, nnz = 0;
+  int device = 0;
+  int sparse = 0;
+  cudaStream_t s = nullptr;
+  cudaEvent_t ev_in = nullptr, ev_out = nullptr;   // order jb_pcaop_apply after / before the caller's stream
+  double* mu = nullptr;          // [d] column means (0 until jb_pcaop_stats)
+  double* var = nullptr;         // [d]
+  // dense operand
+  float* X = nullptr;            // [n, d] as given
+  float* mu32 = nullptr;         // [d]
+  float* x_hi = nullptr;         // [n, ldd] 3xTF32 planes of X - mu
+  float* x_lo = nullptr;
+  long long ldd = 0;
+  double* stat_part = nullptr;   // [PO_STAT_SLABS, d] partial column sums
+  jb::GemmProblem* probs = nullptr;   // one table entry per reduction chunk of a product
+  int n_probs = 0;
+  std::vector<jb::GemmProblem> host_probs;
+  // sparse operand: CSR of X (rp, ci, rv) and CSR of X^T (cp, ri, cv); work items of both directions
+  long long* rp = nullptr; int* ci = nullptr; float* rv = nullptr;
+  long long* cp = nullptr; int* ri = nullptr; float* cv = nullptr;
+  jb::PoItem* items[2] = {nullptr, nullptr};
+  long long n_items[2] = {0, 0};
+  jb::PoLong* longs[2] = {nullptr, nullptr};
+  int n_long[2] = {0, 0};
+  int n_part[2] = {0, 0};
+  // workspaces of width ws_l (grown on demand by jb_pcaop_apply)
+  int ws_l = 0;
+  float* b_hi = nullptr; float* b_lo = nullptr; float* t32 = nullptr;   // dense: planes of B, one chunk's fp32 product
+  double* acc = nullptr;                                                // dense: float64 sum over the chunks
+  double* part = nullptr;                                               // sparse: segment partials
+  double* vpart = nullptr; double* vvec = nullptr;                      // sparse: the l-vector of the rank-1 correction
+};
 
 struct jb_dist {   // one n x n float64 distance matrix on one device (jb_dist_*)
   long long n = 0;
@@ -1878,6 +1913,292 @@ int jb_dist_geodesic(jb_dist* h, int k, double* out) {
   if (out) CU(cudaMemcpyAsync(out, h->D, nn * sizeof(double), cudaMemcpyDeviceToHost, h->s));
   CU(cudaStreamSynchronize(h->s));
   return 0;
+}
+
+// ---------------------------------------------------------------------------------------------- randomized PCA operand (N3)
+
+namespace {
+constexpr long long PO_KCHUNK = 8192;   // dense products: reduction length of one GEMM, accumulated over chunks in float64
+
+int po_check_fits(double need, int device, const char* what) {
+  size_t free_b = 0, total_b = 0;
+  CU(cudaMemGetInfo(&free_b, &total_b));
+  if (need > static_cast<double>(free_b))
+    return fail("%s needs %.2f GB of device memory; %.2f GB of device %d are free", what, need / 1e9, free_b / 1e9, device);
+  return 0;
+}
+
+// CSR consistency: ptr[0] = 0, non-decreasing, ptr[rows] = nnz, every index in [0, cols)
+int po_check_csr(const char* name, long long rows, long long cols, long long nnz, const long long* ptr, const int* idx) {
+  if (ptr[0] != 0) return fail("%s: indptr[0] = %lld, expected 0", name, ptr[0]);
+  if (ptr[rows] != nnz) return fail("%s: indptr[%lld] = %lld, expected nnz = %lld", name, rows, ptr[rows], nnz);
+  for (long long r = 0; r < rows; ++r)
+    if (ptr[r + 1] < ptr[r]) return fail("%s: indptr decreases at row %lld", name, r);
+  for (long long p = 0; p < nnz; ++p)
+    if (idx[p] < 0 || idx[p] >= cols) return fail("%s: index %d at position %lld out of range [0, %lld)", name, idx[p], p, cols);
+  return 0;
+}
+
+// one work item per row, or one per PO_SEG-long segment of a longer row
+void po_items(const long long* ptr, long long rows, std::vector<jb::PoItem>& items, std::vector<jb::PoLong>& longs, int& n_part) {
+  n_part = 0;
+  for (long long r = 0; r < rows; ++r) {
+    const long long b = ptr[r], e = ptr[r + 1];
+    if (e - b <= jb::PO_SEG) { items.push_back({b, e, static_cast<int>(r), -1}); continue; }
+    const int first = n_part;
+    for (long long p = b; p < e; p += jb::PO_SEG) items.push_back({p, p + jb::PO_SEG < e ? p + jb::PO_SEG : e, static_cast<int>(r), n_part++});
+    longs.push_back({static_cast<int>(r), first, n_part - first});
+  }
+}
+
+double po_ws_bytes(const jb_pcaop* h, int l) {
+  const double M = static_cast<double>(h->n > h->d ? h->n : h->d);
+  if (!h->sparse) return M * r4(l) * 4.0 * 3 + M * l * 8.0;
+  const int np = h->n_part[0] > h->n_part[1] ? h->n_part[0] : h->n_part[1];
+  return static_cast<double>(np) * l * 8.0 + (jb::PO_STAT_SLABS + 1.0) * l * 8.0;
+}
+
+void po_free_ws(jb_pcaop* h) {
+  cudaFree(h->b_hi); cudaFree(h->b_lo); cudaFree(h->t32); cudaFree(h->acc); cudaFree(h->part); cudaFree(h->vpart); cudaFree(h->vvec);
+  h->b_hi = h->b_lo = h->t32 = nullptr; h->acc = h->part = h->vpart = h->vvec = nullptr;
+  h->ws_l = 0;
+}
+
+int po_ensure_ws(jb_pcaop* h, int l) {
+  if (l <= h->ws_l) return 0;
+  CU(cudaStreamSynchronize(h->s));   // the old workspaces may still be in use
+  po_free_ws(h);
+  char what[96];
+  snprintf(what, sizeof what, "the workspaces of a width-%d product", l);
+  if (po_check_fits(po_ws_bytes(h, l), h->device, what)) return 1;
+  const size_t M = static_cast<size_t>(h->n > h->d ? h->n : h->d);
+  cudaError_t ce = cudaSuccess;
+  if (!h->sparse) {
+    const size_t pl = M * r4(l);
+    ce = cudaMalloc(&h->b_hi, pl * 4);
+    if (ce == cudaSuccess) ce = cudaMalloc(&h->b_lo, pl * 4);
+    if (ce == cudaSuccess) ce = cudaMalloc(&h->t32, pl * 4);
+    if (ce == cudaSuccess) ce = cudaMalloc(&h->acc, M * l * 8);
+  } else {
+    const int np = h->n_part[0] > h->n_part[1] ? h->n_part[0] : h->n_part[1];
+    ce = cudaMalloc(&h->part, static_cast<size_t>(np > 0 ? np : 1) * l * 8);
+    if (ce == cudaSuccess) ce = cudaMalloc(&h->vpart, static_cast<size_t>(jb::PO_STAT_SLABS) * l * 8);
+    if (ce == cudaSuccess) ce = cudaMalloc(&h->vvec, static_cast<size_t>(l) * 8);
+  }
+  if (ce != cudaSuccess) {
+    po_free_ws(h);
+    return fail("workspaces of a width-%d product: %s", l, cudaGetErrorString(ce));
+  }
+  h->ws_l = l;
+  return 0;
+}
+
+// hi/lo planes of X - mu (fp32 mean subtracted during the split), on the handle's stream
+int po_split_dense(jb_pcaop* h) {
+  jb::k_f64_to_f32<<<static_cast<unsigned>((h->d + 255) / 256), 256, 0, h->s>>>(h->mu, h->d, h->mu32);
+  jb::k_split_tf32<<<static_cast<unsigned>(h->n), 256, 0, h->s>>>(h->X, h->d, h->n, static_cast<int>(h->d), 0, h->mu32, 1.f, 0.f,
+                                                                  h->x_hi, h->x_lo, h->ldd);
+  CU(cudaGetLastError());
+  return 0;
+}
+
+jb_pcaop* po_new(long long n, long long d, int device, int sparse) {
+  jb_pcaop* h = new jb_pcaop();
+  h->n = n; h->d = d; h->device = device; h->sparse = sparse;
+  return h;
+}
+
+// stream, events, mu / var: common to both operand kinds
+cudaError_t po_common_alloc(jb_pcaop* h) {
+  cudaError_t ce = cudaStreamCreateWithFlags(&h->s, cudaStreamNonBlocking);
+  if (ce == cudaSuccess) ce = cudaEventCreateWithFlags(&h->ev_in, cudaEventDisableTiming);
+  if (ce == cudaSuccess) ce = cudaEventCreateWithFlags(&h->ev_out, cudaEventDisableTiming);
+  if (ce == cudaSuccess) ce = cudaMalloc(&h->mu, static_cast<size_t>(h->d) * 8);
+  if (ce == cudaSuccess) ce = cudaMalloc(&h->var, static_cast<size_t>(h->d) * 8);
+  if (ce == cudaSuccess) ce = cudaMemsetAsync(h->mu, 0, static_cast<size_t>(h->d) * 8, h->s);
+  return ce;
+}
+}  // namespace
+
+int jb_pcaop_create_dense(const float* X, long long n, long long d, int device, jb_pcaop** out) {
+  if (!X || !out) return fail("null argument");
+  *out = nullptr;
+  if (n < 1 || d < 1 || n > (1LL << 31) - 1 || d > (1LL << 31) - 32) return fail("bad operand shape %lld x %lld", n, d);
+  CU(cudaSetDevice(device));
+  const long long ldd = r4(static_cast<int>(d));
+  const long long chunks = ((n > d ? n : d) + PO_KCHUNK - 1) / PO_KCHUNK;
+  const double need = 4.0 * n * d + 8.0 * n * ldd + 20.0 * d + 8.0 * jb::PO_STAT_SLABS * d +
+                      static_cast<double>(chunks) * sizeof(jb::GemmProblem);
+  char what[96];
+  snprintf(what, sizeof what, "a dense %lld x %lld PCA operand", n, d);
+  if (po_check_fits(need, device, what)) return 1;
+  jb_pcaop* h = po_new(n, d, device, 0);
+  h->ldd = ldd;
+  h->n_probs = static_cast<int>(chunks);
+  cudaError_t ce = po_common_alloc(h);
+  if (ce == cudaSuccess) ce = cudaMalloc(&h->X, static_cast<size_t>(n) * d * 4);
+  if (ce == cudaSuccess) ce = cudaMalloc(&h->x_hi, static_cast<size_t>(n) * ldd * 4);
+  if (ce == cudaSuccess) ce = cudaMalloc(&h->x_lo, static_cast<size_t>(n) * ldd * 4);
+  if (ce == cudaSuccess) ce = cudaMalloc(&h->mu32, static_cast<size_t>(d) * 4);
+  if (ce == cudaSuccess) ce = cudaMalloc(&h->stat_part, static_cast<size_t>(jb::PO_STAT_SLABS) * d * 8);
+  if (ce == cudaSuccess) ce = cudaMalloc(&h->probs, static_cast<size_t>(chunks) * sizeof(jb::GemmProblem));
+  if (ce == cudaSuccess) ce = cudaMemcpyAsync(h->X, X, static_cast<size_t>(n) * d * 4, cudaMemcpyHostToDevice, h->s);
+  if (ce != cudaSuccess) {
+    jb_pcaop_destroy(h);
+    return fail("dense PCA operand of %lld x %lld: %s", n, d, cudaGetErrorString(ce));
+  }
+  if (po_split_dense(h)) { jb_pcaop_destroy(h); return 1; }
+  ce = cudaStreamSynchronize(h->s);
+  if (ce != cudaSuccess) {
+    jb_pcaop_destroy(h);
+    return fail("dense PCA operand of %lld x %lld: %s", n, d, cudaGetErrorString(ce));
+  }
+  *out = h;
+  return 0;
+}
+
+int jb_pcaop_create_sparse(long long n, long long d, long long nnz, const long long* row_ptr, const int* col_idx,
+                           const float* row_val, const long long* col_ptr, const int* row_idx, const float* col_val,
+                           int device, jb_pcaop** out) {
+  if (!out || !row_ptr || !col_ptr || (nnz > 0 && (!col_idx || !row_val || !row_idx || !col_val))) return fail("null argument");
+  *out = nullptr;
+  if (n < 1 || d < 1 || n > (1LL << 31) - 1 || d > (1LL << 31) - 1 || nnz < 0) return fail("bad operand shape %lld x %lld, %lld nonzeros", n, d, nnz);
+  if (po_check_csr("CSR of X", n, d, nnz, row_ptr, col_idx) || po_check_csr("CSR of X^T", d, n, nnz, col_ptr, row_idx)) return 1;
+  std::vector<jb::PoItem> items[2];
+  std::vector<jb::PoLong> longs[2];
+  int n_part[2];
+  po_items(row_ptr, n, items[0], longs[0], n_part[0]);
+  po_items(col_ptr, d, items[1], longs[1], n_part[1]);
+  CU(cudaSetDevice(device));
+  const double need = 8.0 * (n + 1) + 8.0 * (d + 1) + 16.0 * nnz + 16.0 * d +
+                      sizeof(jb::PoItem) * static_cast<double>(items[0].size() + items[1].size()) +
+                      sizeof(jb::PoLong) * static_cast<double>(longs[0].size() + longs[1].size());
+  char what[128];
+  snprintf(what, sizeof what, "a sparse %lld x %lld PCA operand with %lld nonzeros", n, d, nnz);
+  if (po_check_fits(need, device, what)) return 1;
+  jb_pcaop* h = po_new(n, d, device, 1);
+  h->nnz = nnz;
+  cudaError_t ce = po_common_alloc(h);
+  auto up = [&](auto** dst, const auto* src, size_t count) {
+    if (ce != cudaSuccess) return;
+    ce = cudaMalloc(dst, (count ? count : 1) * sizeof(**dst));
+    if (ce == cudaSuccess && count) ce = cudaMemcpyAsync(*dst, src, count * sizeof(**dst), cudaMemcpyHostToDevice, h->s);
+  };
+  up(&h->rp, row_ptr, static_cast<size_t>(n) + 1);
+  up(&h->ci, col_idx, static_cast<size_t>(nnz));
+  up(&h->rv, row_val, static_cast<size_t>(nnz));
+  up(&h->cp, col_ptr, static_cast<size_t>(d) + 1);
+  up(&h->ri, row_idx, static_cast<size_t>(nnz));
+  up(&h->cv, col_val, static_cast<size_t>(nnz));
+  for (int t = 0; t < 2; ++t) {
+    h->n_items[t] = static_cast<long long>(items[t].size());
+    h->n_long[t] = static_cast<int>(longs[t].size());
+    h->n_part[t] = n_part[t];
+    up(&h->items[t], items[t].data(), items[t].size());
+    up(&h->longs[t], longs[t].data(), longs[t].size());
+  }
+  if (ce == cudaSuccess) ce = cudaStreamSynchronize(h->s);   // the host vectors above go out of scope
+  if (ce != cudaSuccess) {
+    jb_pcaop_destroy(h);
+    return fail("sparse PCA operand of %lld x %lld: %s", n, d, cudaGetErrorString(ce));
+  }
+  *out = h;
+  return 0;
+}
+
+int jb_pcaop_stats(jb_pcaop* h, double* mean, double* var) {
+  if (!h) return fail("null argument");
+  CU(cudaSetDevice(h->device));
+  const long long n = h->n, d = h->d;
+  if (h->sparse) {
+    jb::k_csc_stats<<<static_cast<unsigned>((d * 32 + 255) / 256), 256, 0, h->s>>>(h->cp, h->cv, d, n, h->mu, h->var);
+  } else {
+    const long long per = (n + jb::PO_STAT_SLABS - 1) / jb::PO_STAT_SLABS;
+    const dim3 g(static_cast<unsigned>((d + 127) / 128), jb::PO_STAT_SLABS);
+    const unsigned gs = static_cast<unsigned>((d + 255) / 256);
+    jb::k_col_sums<<<g, 128, 0, h->s>>>(h->X, n, d, per, h->stat_part);
+    jb::k_sum_parts<<<gs, 256, 0, h->s>>>(h->stat_part, jb::PO_STAT_SLABS, d, static_cast<double>(n), h->mu);
+    jb::k_col_sqdev<<<g, 128, 0, h->s>>>(h->X, n, d, per, h->mu, h->stat_part);
+    jb::k_sum_parts<<<gs, 256, 0, h->s>>>(h->stat_part, jb::PO_STAT_SLABS, d, static_cast<double>(n), h->var);
+    if (po_split_dense(h)) return 1;
+  }
+  CU(cudaGetLastError());
+  if (mean) CU(cudaMemcpyAsync(mean, h->mu, static_cast<size_t>(d) * 8, cudaMemcpyDeviceToHost, h->s));
+  if (var) CU(cudaMemcpyAsync(var, h->var, static_cast<size_t>(d) * 8, cudaMemcpyDeviceToHost, h->s));
+  CU(cudaStreamSynchronize(h->s));
+  return 0;
+}
+
+int jb_pcaop_apply(jb_pcaop* h, int trans, const float* B, int l, float* Y, void* stream) {
+  if (!h || !B || !Y) return fail("null argument");
+  if (trans != 0 && trans != 1) return fail("trans must be 0 or 1, not %d", trans);
+  if (l < 1 || l > 65536) return fail("bad product width %d (1 .. 65536)", l);
+  CU(cudaSetDevice(h->device));
+  if (po_ensure_ws(h, l)) return 1;
+  cudaStream_t cs = static_cast<cudaStream_t>(stream);
+  CU(cudaEventRecord(h->ev_in, cs));
+  CU(cudaStreamWaitEvent(h->s, h->ev_in, 0));
+  const long long K = trans ? h->n : h->d, M = trans ? h->d : h->n;   // B [K, l], Y [M, l]
+  if (h->sparse) {
+    // the l-vector of the rank-1 correction: mu^T B (trans 0, a = 1) or 1^T B (trans 1, a = mu), in a fixed order
+    const long long per = (K + jb::PO_STAT_SLABS - 1) / jb::PO_STAT_SLABS;
+    jb::k_wcolsum<<<dim3(static_cast<unsigned>((l + 127) / 128), jb::PO_STAT_SLABS), 128, 0, h->s>>>(B, K, l, per, trans ? nullptr : h->mu, h->vpart);
+    jb::k_sum_parts<<<static_cast<unsigned>((l + 255) / 256), 256, 0, h->s>>>(h->vpart, jb::PO_STAT_SLABS, l, 1.0, h->vvec);
+    const double* a = trans ? h->mu : nullptr;
+    const int* idx = trans ? h->ri : h->ci;
+    const float* val = trans ? h->cv : h->rv;
+    const dim3 g(static_cast<unsigned>((h->n_items[trans] + jb::PO_WARPS - 1) / jb::PO_WARPS), static_cast<unsigned>((l + jb::PO_SLAB - 1) / jb::PO_SLAB));
+    jb::k_csr_dense<<<g, jb::PO_WARPS * 32, 0, h->s>>>(h->items[trans], h->n_items[trans], idx, val, B, l, a, h->vvec, Y, h->part);
+    if (h->n_long[trans]) {
+      const long long t = static_cast<long long>(h->n_long[trans]) * l;
+      jb::k_seg_finish<<<static_cast<unsigned>((t + 255) / 256), 256, 0, h->s>>>(h->longs[trans], h->n_long[trans], h->part, l, a, h->vvec, Y);
+    }
+  } else {
+    // Y = Xc B (trans 0: A = the [n, d] planes, K-major) or Xc^T B (trans 1: the same planes read MN-major); B [K, l] is
+    // MN-major. One 3xTF32 GEMM per PO_KCHUNK slice of K, each added to a float64 accumulator, then one rounding to fp32.
+    const int ldl = r4(l);
+    jb::k_split_tf32<<<static_cast<unsigned>(K), 256, 0, h->s>>>(B, l, K, l, 2, nullptr, 1.f, 0.f, h->b_hi, h->b_lo, ldl);
+    CU(cudaMemsetAsync(h->acc, 0, static_cast<size_t>(M) * l * 8, h->s));
+    const int chunks = static_cast<int>((K + PO_KCHUNK - 1) / PO_KCHUNK);
+    const int bn = l <= 32 ? 32 : 64;
+    h->host_probs.assign(static_cast<size_t>(chunks), jb::GemmProblem{});
+    for (int c = 0; c < chunks; ++c) {
+      const long long k0 = c * PO_KCHUNK, kc = K - k0 < PO_KCHUNK ? K - k0 : PO_KCHUNK;
+      const long long a_off = trans ? k0 * h->ldd : k0;
+      jb::GemmProblem& g = h->host_probs[static_cast<size_t>(c)];
+      int rc = jb::gemm_problem_fill(&g, h->x_hi + a_off, static_cast<int>(h->ldd), trans, h->b_hi + k0 * ldl, ldl, 1, h->t32, ldl,
+                                     static_cast<int>(M), l, static_cast<int>(kc), bn, jb::EPI_STORE, nullptr, 0.f, 0, 0,
+                                     h->x_lo + a_off, h->b_lo + k0 * ldl);
+      if (rc) return fail("PCA operand tensor map encode failed (%d)", rc);
+      jb::gemm_table_finalize(&g, 1);
+    }
+    CU(cudaMemcpyAsync(h->probs, h->host_probs.data(), static_cast<size_t>(chunks) * sizeof(jb::GemmProblem), cudaMemcpyHostToDevice, h->s));
+    for (int c = 0; c < chunks; ++c) {
+      const jb::GemmProblem& g = h->host_probs[static_cast<size_t>(c)];
+      CU(jb::gemm_launch(h->probs + c, 1, g.tiles_m * g.tiles_n, h->s));
+      jb::k_acc_f64<<<static_cast<unsigned>(M), 256, 0, h->s>>>(h->t32, ldl, h->acc, l);
+    }
+    jb::k_f64_to_f32<<<static_cast<unsigned>((M * l + 255) / 256), 256, 0, h->s>>>(h->acc, M * l, Y);
+  }
+  CU(cudaGetLastError());
+  CU(cudaEventRecord(h->ev_out, h->s));
+  CU(cudaStreamWaitEvent(cs, h->ev_out, 0));
+  return 0;
+}
+
+void jb_pcaop_destroy(jb_pcaop* h) {
+  if (!h) return;
+  cudaSetDevice(h->device);
+  if (h->s) cudaStreamSynchronize(h->s);
+  po_free_ws(h);
+  cudaFree(h->mu); cudaFree(h->var); cudaFree(h->X); cudaFree(h->mu32); cudaFree(h->x_hi); cudaFree(h->x_lo);
+  cudaFree(h->stat_part); cudaFree(h->probs);
+  cudaFree(h->rp); cudaFree(h->ci); cudaFree(h->rv); cudaFree(h->cp); cudaFree(h->ri); cudaFree(h->cv);
+  for (int t = 0; t < 2; ++t) { cudaFree(h->items[t]); cudaFree(h->longs[t]); }
+  if (h->ev_in) cudaEventDestroy(h->ev_in);
+  if (h->ev_out) cudaEventDestroy(h->ev_out);
+  if (h->s) cudaStreamDestroy(h->s);
+  delete h;
 }
 
 long long jb_debug_read(jb_engine* e, const char* name, float* out, long long cap) {

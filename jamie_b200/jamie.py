@@ -203,8 +203,11 @@ class JAMIE(UnionCom):
         assert sampler in ('auto', 'reference', 'fast'), f"sampler must be 'auto', 'reference' or 'fast', not {sampler!r}"
         self.sampler = sampler
         # pca_fit (not in the reference): 'gpu' = column sums + Gram matrix on the GPU, d x d eigensolver on the host (sklearn's
-        # covariance_eigh algorithm, exact PCA); 'sklearn' = the reference's host call PCA(n_components).fit_transform(data).
-        assert pca_fit in ('gpu', 'sklearn'), f"pca_fit must be 'gpu' or 'sklearn', not {pca_fit!r}"
+        # covariance_eigh algorithm, exact PCA); 'sklearn' = the reference's host call PCA(n_components).fit_transform(data);
+        # 'randomized' = sklearn's randomized solver with its products on the GPU (wide and sparse inputs: no d x d matrix,
+        # a scipy.sparse input is never densified; seeded with manual_seed).
+        assert pca_fit in ('gpu', 'sklearn', 'randomized'), \
+            f"pca_fit must be 'gpu', 'sklearn' or 'randomized', not {pca_fit!r}"
         self.pca_fit = pca_fit
         # distances (not in the reference): 'host' = compute_distances with the reference's sklearn / scipy calls; 'gpu' = the
         # same distances from the jb_dist kernels on the engine's device (correspondence.gpu_distance_function; a scipy.sparse
@@ -396,6 +399,13 @@ class JAMIE(UnionCom):
                         fit_engine = Engine([8, 8], 2, 8, 0.0, device=dev0)
                     pca, sample = pca_fit.fit_transform(fit_engine, data if pca_fit.is_sparse(data) else np.asarray(data),
                                                         dim, rank, world)
+                elif self.pca_fit == 'randomized':
+                    # every rank runs the same seeded fit on all rows (no engine needed: the operand owns its device copy)
+                    from . import pca_fit
+                    dev0 = self._cuda_index()
+                    torch.cuda.set_device(dev0)
+                    pca, sample = pca_fit.randomized_fit_transform(data if pca_fit.is_sparse(data) else np.asarray(data), dim,
+                                                                   seed=self.manual_seed, device=dev0)
                 else:
                     pca = make_pca(dim)
                     sample = pca.fit_transform(data)
