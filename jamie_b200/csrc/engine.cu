@@ -113,7 +113,6 @@ struct jb_engine {
   float* xg[8]{}; unsigned int* xf[8]{}; float* xmc = nullptr; int xrank = 0, xworld = 0; long long x_adam0 = 0;   // in-kernel exchange (jb_set_exchange)
   float* grad_own = nullptr;        // the engine's own gradient buffer while a caller-owned one is in use (jb_set_grad_buffer)
   __half* theta_eval_h = nullptr;   // fp16 copy of the folded inference weights (operands of the fp16 layers of the chain)
-  bool eval_f16 = true;             // JB_EVAL_F16=0: the whole chain in TF32 with fp32 activations
   __half *theta_hi = nullptr, *theta_lo = nullptr;   // fp16 operand planes of theta (same element offsets)
   float* state_slab = nullptr;   // one allocation: theta | adam_m | adam_v | theta_hi, theta_lo
   size_t slab_bytes = 0;
@@ -136,7 +135,6 @@ struct jb_engine {
   jb::Ctl* ctl = nullptr;
   double* norm_part = nullptr;
   float *norm_tile = nullptr, *norm_small = nullptr;   // fused clip norm (stepk.cuh)
-  int norm_fuse = 1;                                   // JB_NORM_FUSE=0: always sweep the gradient buffer
   int norm_tile_cap = 0;
   unsigned int* bar = nullptr;          // grid barrier counters of k_step: [0] and [32], used by alternate launches
   int bar_parity = 0;
@@ -157,15 +155,8 @@ struct jb_engine {
   jb::StepCtx& h_ctx_ref() { return h_prm->cx; }
   int step_B = 0;
   int grid = 132;            // CTAs of k_step: HG_CLUSTER x the co-resident clusters (33 x 4 on B200; set in jb_create)
-  int fuse_enabled = 1;      // JB_FUSE=0: BatchNorm / reconstruction / reparameterisation as separate phases (the B > 512 path)
   int fused = 0;             // the current step tables use the cluster-fused tails
-  int merge_latent = 1;      // JB_MERGE_LATENT=0: LATLOSS / LATFIN as separate phases even without F
-  int fuse_ks = 1;           // JB_FUSE_KS=0: HEADS / DG3 as one CTA per M tile instead of K split over the cluster
   int accumulate = 0, accumulate_dev = 0;
-  int wgrad_mode = jb::HG_MEDIUM;
-  int fwd_mode = -1;                // forward / dgrad GEMM mode: -1 = by K (see build_step), else forced (JB_FWD_MODE=precise | medium)
-  int wgrad_bn = 256;
-  int max_ksplit = 8;
   float gs = 1.f;
   // Host-batch steps (data resident on the host): two slots so that the copies of batch k + 1 run while step k computes.
   struct HostPin* h_pin = nullptr;   // pinned: constants, per-slot kl / losses / indices
@@ -173,13 +164,10 @@ struct jb_engine {
   cudaEvent_t ev_h2d[2]{}, ev_slot_free[2]{}, ev_loss[2]{};
   bool slot_used[2]{};
   int hb_slot = 0, hb_oldest = 0, hb_outstanding = 0;
-  int precision_fast = 0;    // JB_PRECISION=f16: single-pass fp16 everywhere (no parity claim)
   int num_sms = 148;
   // eval
   bool eval_dirty = true;
-  int eval_chunk = 8192;     // rows per pass of the folded chain (JB_EVAL_CHUNK); activations of a chunk stay in L2
-  int eval_bn256_min = 256;  // layers at least this wide use 256-column tiles (JB_EVAL_BN256_MIN)
-  bool eval_persist = true;  // inference chain on the persistent GEMM (JB_EVAL_PERSIST=0: one tile per CTA)
+  int eval_chunk = 8192;     // rows per pass of the folded chain (set in jb_create); activations of a chunk stay in L2
   float *ev_a = nullptr, *ev_b = nullptr, *ev_in = nullptr, *ev_out = nullptr;
   jb::GemmProblem* d_ev_probs = nullptr;
   int ev_probs_cap = 0;
@@ -331,22 +319,17 @@ int build_step(jb_engine* e, int B) {
     for (int k = 0; k < 4; ++k) wmax = fmaxf(wmax, fabsf(e->cfg.loss_w[k]));
     const int ex = static_cast<int>(ceil(log2(static_cast<double>(B) * Dm))) - static_cast<int>(ceil(log2(static_cast<double>(wmax))));
     e->gs = ldexpf(1.f, ex < 0 ? 0 : (ex > 30 ? 30 : ex));
-    if (const char* pv = getenv("JB_LOSS_SCALE_LOG2")) e->gs = ldexpf(1.f, atoi(pv));
   }
   const float inv_gs = 1.f / e->gs;
   // Forward / dgrad mode by reduction length: the tensor core adds products into its fp32 accumulator with truncation, a
   // bias that grows with the number of accumulation steps. Up to K = 1024 (64 steps) three undrained passes (HG_MEDIUM)
   // stay at 7e-6 of the fp32 oracle at the headline shape and save 9 us per step; longer reductions (2000-wide inputs
   // without PCA: measured 6e-4 undrained) keep the drained HG_PRECISE mode.
-  auto fmode_for = [&](int K) {
-    if (e->precision_fast) return static_cast<int>(jb::HG_SINGLE);
-    if (e->fwd_mode >= 0) return e->fwd_mode;
-    return static_cast<int>(K <= 1024 ? jb::HG_MEDIUM : jb::HG_PRECISE);
-  };
-  const int wmode = e->precision_fast ? jb::HG_SINGLE : e->wgrad_mode;
+  auto fmode_for = [](int K) { return static_cast<int>(K <= 1024 ? jb::HG_MEDIUM : jb::HG_PRECISE); };
   std::vector<std::vector<StageSpec>> st(jb::SK_NUM_GEMM);
-  // Cluster-fused tails need all rows of a column block in one cluster: B <= HG_CLUSTER M tiles.
-  const bool fused = e->fuse_enabled && B <= jb::HG_CLUSTER * jb::HG_BM;
+  // Cluster-fused tails need all rows of a column block in one cluster: B <= HG_CLUSTER M tiles. Larger batches run
+  // BatchNorm / reconstruction / reparameterisation as separate slab phases.
+  const bool fused = B <= jb::HG_CLUSTER * jb::HG_BM;
   e->fused = fused ? 1 : 0;
   const int nclusters = e->grid / jb::HG_CLUSTER;
   // N tile of the forward / dgrad stages: 64 columns, or 32 when the 64-wide column blocks of both modalities would leave
@@ -366,7 +349,7 @@ int build_step(jb_engine* e, int B) {
         static const int bn_layer[6] = {0, 1, -1, 2, 3, -1};
         if (bn_layer[stage] >= 0) { sp.fuse = jb::FUSE_BN_FWD; sp.fuse_arg = bn_layer[stage] * 2 + i; }
         else if (stage == 5) { sp.fuse = jb::FUSE_REC; sp.fuse_arg = i; }
-        else if (stage == 2 && 2 * L <= 64) { sp.fuse = jb::FUSE_HEADS; sp.fuse_arg = i; sp.fuse_ks = e->fuse_ks && n_in >= 8 * jb::HG_BK; }
+        else if (stage == 2 && 2 * L <= 64) { sp.fuse = jb::FUSE_HEADS; sp.fuse_arg = i; sp.fuse_ks = n_in >= 8 * jb::HG_BK; }
         // narrow column blocks only pay where the main loop is long (K >= 256); short-K stages keep 64
         if (stage != 2 && n_out > 32 && n_in >= 256) sp.bn = stage == 0 || stage == 4 ? fbn2(2 * e->D[0], 2 * e->D[1]) : fbn2(e->D[0], e->D[1]);
       }
@@ -382,7 +365,7 @@ int build_step(jb_engine* e, int B) {
     auto dgrad = [&](int stage, HPlanes dY, int lddy, const Seg& s, jb::Parts* out, int lddx, int n_out, int n_in) {
       StageSpec sp{dY, lddy, 0, W(s), s.ld, 1, out, nullptr, lddx, B, n_in, n_out, fbn(n_in), fmode_for(n_out), jb::EPI_STORE, nullptr, 1.f, 0, -1};
       if (fused && stage == 8) {   // d c: the LATBC phase becomes the tail (no F, one column block)
-        if (e->f_dense == nullptr && e->merge_latent && L <= 64) { sp.fuse = jb::FUSE_LATBC; sp.fuse_arg = i; sp.fuse_ks = e->fuse_ks && n_out >= 8 * jb::HG_BK; }
+        if (e->f_dense == nullptr && L <= 64) { sp.fuse = jb::FUSE_LATBC; sp.fuse_arg = i; sp.fuse_ks = n_out >= 8 * jb::HG_BK; }
       } else if (fused) {   // the dgrad result feeds a BatchNorm backward: stage 6 -> dec2, 7 -> dec1, 9 -> enc2, 10 -> enc1
         const int k = stage == 6 ? 3 : (stage == 7 ? 2 : (stage == 9 ? 1 : 0));
         sp.fuse = jb::FUSE_BN_BWD; sp.fuse_arg = k * 2 + i;
@@ -401,8 +384,8 @@ int build_step(jb_engine* e, int B) {
   // items at the headline shape) and d Wmv = d[mu|logvar]^T h2 beside DGH, on CTAs those phases leave idle; WGRAD is then
   // exactly one work item per CTA (128 items of 128 x 256 on 132 CTAs).
   auto wgrad = [&](HPlanes dY, int lddy, HPlanes X, int ldx, const Seg& s, int n_out, int n_in, int dyn, int stage = 11) {
-    int bn = n_in <= 32 ? 32 : (n_in <= 64 || stage != 11 ? 64 : (n_in >= 256 && e->wgrad_bn >= 256 ? 256 : 128));
-    st[stage].push_back(StageSpec{dY, lddy, 1, X, ldx, 1, nullptr, G + s.off, s.ld, n_out, n_in, B, bn, wmode, jb::EPI_STORE, nullptr, inv_gs, 1, dyn});
+    int bn = n_in <= 32 ? 32 : (n_in <= 64 || stage != 11 ? 64 : (n_in >= 256 ? 256 : 128));
+    st[stage].push_back(StageSpec{dY, lddy, 1, X, ldx, 1, nullptr, G + s.off, s.ld, n_out, n_in, B, bn, jb::HG_MEDIUM, jb::EPI_STORE, nullptr, inv_gs, 1, dyn});
   };
   for (int i = 0; i < 2; ++i) { ModActs& a = e->act[i]; ModSegs& m = e->ms[i]; const int D = e->D[i];
     // encoder-side gradients carry the dynamic scale s_b of d[mu | logvar] (dyn 1); dW3's B operand is the c planes (dyn 0)
@@ -410,7 +393,8 @@ int build_step(jb_engine* e, int B) {
     wgrad(a.dy2, a.ldD, a.h1, a.ld2D, m.W2, D, 2 * D, 1); wgrad(a.dy1, a.ld2D, a.xp, a.ldD, m.W1, 2 * D, D, 1); }
   for (int i = 0; i < 2; ++i) { ModActs& a = e->act[i]; ModSegs& m = e->ms[i]; const int D = e->D[i];
     wgrad(a.dmp, e->ldmv, a.h2, a.ldD, m.Wmv, 2 * L, D, 1, 9); wgrad(a.dy3, a.ldD, a.cp, e->LP, m.W3, D, L, 0, 8); }
-  // split-K factor per problem: fill the grid, at least two k-blocks per partial
+  // split-K factor per problem: fill the grid, at least two k-blocks per partial, at most kMaxKsplit partials
+  constexpr int kMaxKsplit = 8;
   size_t parts_bytes = 0;
   std::vector<std::vector<int>> ks(jb::SK_NUM_GEMM);
   for (int g = 0; g < jb::SK_NUM_GEMM; ++g) {
@@ -422,7 +406,7 @@ int build_step(jb_engine* e, int B) {
         const int kb = (s.K + jb::HG_BK - 1) / jb::HG_BK;
         k = s.fuse ? (s.fuse_ks ? jb::HG_CLUSTER : 1) : e->grid / (tiles > 0 ? tiles : 1);
         if (k > kb / 2) k = kb / 2;
-        if (k > e->max_ksplit) k = e->max_ksplit;
+        if (k > kMaxKsplit) k = kMaxKsplit;
         if (k < 1) k = 1;
         parts_bytes = ((parts_bytes + 255) & ~size_t(255)) + static_cast<size_t>(k) * s.M * s.ldc * 4;
       }
@@ -541,7 +525,6 @@ int build_step(jb_engine* e, int B) {
     }
   }
   cx.norm_tile = e->norm_tile; cx.norm_small = e->norm_small; cx.n_norm_tile = n_norm_tile;
-  cx.norm_fuse = e->norm_fuse ? 1 : 0;
   {
     int nr = 0;
     auto rng = [&](const Seg& sg) { cx.norm_rng[nr][0] = static_cast<int>(sg.off); cx.norm_rng[nr][1] = sg.cols; ++nr; };
@@ -552,14 +535,14 @@ int build_step(jb_engine* e, int B) {
     }
     cx.n_norm_rng = nr;
   }
-  cx.merge_latent = (e->f_dense == nullptr && e->merge_latent) ? 1 : 0;
+  cx.merge_latent = e->f_dense == nullptr ? 1 : 0;
   if (cx.merge_latent) cx.phase_mask &= ~((1ull << jb::PH_LATLOSS) | (1ull << jb::PH_LATFIN));
   if (e->h_probs[cx.gph[8].first].fuse == jb::FUSE_LATBC) cx.phase_mask &= ~(1ull << jb::PH_LATBC);
   cx.p_diag = e->p_diag; cx.p_dense = e->p_dense; cx.f_dense = e->f_dense; cx.pn1 = e->pn1;
   cx.corr = e->corr; cx.corr_t = e->corr_t; cx.fblk = e->fblk; cx.fblk_t = e->fblk_t;
   cx.pf_ratio = e->cfg.pf_ratio; cx.f_present = e->f_dense != nullptr;
   // the row shortcut of COMBINE / LATBZ exists where GATHER builds the blocks with sk_corr_row_diag (same condition as there)
-  cx.corr_hint = (e->p_diag != nullptr && e->p_dense == nullptr && e->f_dense == nullptr && !getenv("JB_NO_CORR_HINT")) ? e->corr_hint : nullptr;
+  cx.corr_hint = (e->p_diag != nullptr && e->p_dense == nullptr && e->f_dense == nullptr) ? e->corr_hint : nullptr;
   cx.lat_r = e->lat_r; cx.rowpart = e->rowpart; cx.lat_coef = e->lat_coef; cx.cosine = e->cosine;
   cx.cmax_part = e->cmax_part; cx.dmax_part = e->dmax_part; cx.dyn = e->dyn;
   {
@@ -582,12 +565,6 @@ int build_step(jb_engine* e, int B) {
   cx.xrank = e->xrank; cx.xworld = e->xworld; cx.xmc = e->xworld > 1 ? e->xmc : nullptr; cx.x_adam0 = e->x_adam0;
   cx.xdbg = getenv("JB_XCHG_DBG") ? atoi(getenv("JB_XCHG_DBG")) : 0;
   cx.xfence = (getenv("JB_XCHG_FENCE") && strcmp(getenv("JB_XCHG_FENCE"), "sys") == 0) ? 1 : 0;
-  cx.adam_stream = 1;
-  if (const char* pv = getenv("JB_ADAM_STREAM")) cx.adam_stream = atoi(pv);
-  cx.prefetch_state = 0;   // measured: WGRAD +9.4 us (the prefetch competes with the operand loads), ADAM only -3.5 us
-  if (const char* pv = getenv("JB_PREFETCH_STATE")) cx.prefetch_state = atoi(pv) != 0;
-  cx.dbg_repeat = 1;
-  if (const char* pv = getenv("JB_DBG_REPEAT")) { if (atoi(pv) >= 1) cx.dbg_repeat = atoi(pv); }
   e->step_B = B;
   return 0;
 }
@@ -654,7 +631,8 @@ int prepare_eval(jb_engine* e, cudaStream_t s) {
       ++e->launches;
     }
   }
-  if (e->eval_f16) { jb::k_to_half<<<296, 256, 0, s>>>(e->theta_eval, e->theta_eval_h, e->n_flat); ++e->launches; }
+  jb::k_to_half<<<296, 256, 0, s>>>(e->theta_eval, e->theta_eval_h, e->n_flat);
+  ++e->launches;
   CU(cudaGetLastError());
   e->eval_dirty = false;
   return 0;
@@ -669,75 +647,41 @@ int run_chain(jb_engine* e, int from, int to, const float* in, int ld_in, int ro
   ModSegs& mf = e->ms[from];
   const int Df = e->D[from];
   std::vector<GemmProblem> tab;
-  if (e->eval_persist && e->eval_f16) {
-    // fp16 chain: the wide layers exchange fp16 activations and read fp16 weights (half the operand bytes); the first
-    // layer of each half reads fp32 (the caller's rows, the fp32 embedding) as TF32; embeddings and outputs stay fp32
-    const __half* Th = e->theta_eval_h;
-    __half* hA = reinterpret_cast<__half*>(bufA);
-    __half* hB = reinterpret_cast<__half*>(bufB);
-    auto addc = [&](const void* A, int lda, const Seg& Wt, const Seg& bt, void* C, int ldc, int N, int K, int epi, int f16_ops, int out_f16) {
-      GemmProblem g;
-      int bn = N <= 32 ? 32 : (N <= 64 ? 64 : (N >= e->eval_bn256_min ? 256 : 128));
-      if (out_f16 && bn < 64) bn = 64;
-      const void* Bw = f16_ops ? static_cast<const void*>(Th + Wt.off) : static_cast<const void*>(T + Wt.off);
-      int rc = jb::gemm_chain_problem_fill(&g, A, lda, Bw, Wt.ld, C, ldc, rows, N, K, bn, epi, T + bt.off, jb::LRELU, f16_ops, out_f16);
-      if (rc) return fail("eval tensor map encode failed (%d)", rc);
-      jb::gemm_table_finalize(&g, 1);
-      tab.push_back(g);
-      return 0;
-    };
-    const int h2f = r8(2 * Df), hf = r8(Df);
-    if (addc(in, ld_in, mf.W1, mf.b1, hA, h2f, 2 * Df, Df, jb::EPI_BIAS_LRELU, 0, 1)) return 1;
-    if (addc(hA, h2f, mf.W2, mf.b2, hB, hf, Df, 2 * Df, jb::EPI_BIAS_LRELU, 1, 1)) return 1;
-    if (to < 0) {
-      if (addc(hB, hf, mf.Wmv, mf.bmv, out, ld_out, L, Df, jb::EPI_BIAS, 1, 0)) return 1;
-    } else {
-      ModSegs& mt = e->ms[to];
-      const int Dt = e->D[to];
-      const int h2t = r8(2 * Dt), ht = r8(Dt);
-      if (addc(hB, hf, mf.Wmv, mf.bmv, bufA, e->LP, L, Df, jb::EPI_BIAS, 1, 0)) return 1;
-      if (addc(bufA, e->LP, mt.W3, mt.b3, hB, ht, Dt, L, jb::EPI_BIAS_LRELU, 0, 1)) return 1;
-      if (addc(hB, ht, mt.W4, mt.b4, hA, h2t, 2 * Dt, Dt, jb::EPI_BIAS_LRELU, 1, 1)) return 1;
-      if (addc(hA, h2t, mt.W5, mt.b5, out, ld_out, Dt, 2 * Dt, jb::EPI_BIAS, 1, 0)) return 1;
-    }
-    CU(cudaMemcpyAsync(d_tab, tab.data(), tab.size() * sizeof(GemmProblem), cudaMemcpyHostToDevice, s));
-    for (size_t k = 0; k < tab.size(); ++k) {
-      CU(jb::gemm_launch_persistent(d_tab + k, tab[k], e->num_sms, s, k > 0));
-      ++e->launches;
-    }
-    return 0;
-  }
-  auto add = [&](const float* A, int lda, const Seg& Wt, const Seg& bt, int n_rows_w, float* C, int ldc, int N, int K, int epi) {
+  // fp16 chain: the wide layers exchange fp16 activations and read fp16 weights (half the operand bytes); the first
+  // layer of each half reads fp32 (the caller's rows, the fp32 embedding) as TF32; embeddings and outputs stay fp32
+  const __half* Th = e->theta_eval_h;
+  __half* hA = reinterpret_cast<__half*>(bufA);
+  __half* hB = reinterpret_cast<__half*>(bufB);
+  auto addc = [&](const void* A, int lda, const Seg& Wt, const Seg& bt, void* C, int ldc, int N, int K, int epi, int f16_ops, int out_f16) {
     GemmProblem g;
-    (void)n_rows_w;
-    int bn = N <= 32 ? 32 : (N <= 64 ? 64 : (N >= e->eval_bn256_min ? 256 : 128));   // single pass: wide tiles, fewer operand bytes per output
-    int rc = jb::gemm_problem_fill(&g, A, lda, 0, T + Wt.off, Wt.ld, 0, C, ldc, rows, N, K, bn, epi, T + bt.off, jb::LRELU, 0);
+    int bn = N <= 32 ? 32 : (N <= 64 ? 64 : (N >= 256 ? 256 : 128));
+    if (out_f16 && bn < 64) bn = 64;
+    const void* Bw = f16_ops ? static_cast<const void*>(Th + Wt.off) : static_cast<const void*>(T + Wt.off);
+    int rc = jb::gemm_chain_problem_fill(&g, A, lda, Bw, Wt.ld, C, ldc, rows, N, K, bn, epi, T + bt.off, jb::LRELU, f16_ops, out_f16);
     if (rc) return fail("eval tensor map encode failed (%d)", rc);
-    if (e->eval_persist && (rc = jb::gemm_problem_set_store_map(&g))) return fail("eval output tensor map encode failed (%d)", rc);
     jb::gemm_table_finalize(&g, 1);
     tab.push_back(g);
     return 0;
   };
-  const int ld2f = r4(2 * Df), ldf = r4(Df);
-  if (add(in, ld_in, mf.W1, mf.b1, 0, bufA, ld2f, 2 * Df, Df, jb::EPI_BIAS_LRELU)) return 1;
-  if (add(bufA, ld2f, mf.W2, mf.b2, 0, bufB, ldf, Df, 2 * Df, jb::EPI_BIAS_LRELU)) return 1;
+  const int h2f = r8(2 * Df), hf = r8(Df);
+  if (addc(in, ld_in, mf.W1, mf.b1, hA, h2f, 2 * Df, Df, jb::EPI_BIAS_LRELU, 0, 1)) return 1;
+  if (addc(hA, h2f, mf.W2, mf.b2, hB, hf, Df, 2 * Df, jb::EPI_BIAS_LRELU, 1, 1)) return 1;
   if (to < 0) {
-    if (add(bufB, ldf, mf.Wmv, mf.bmv, 0, out, ld_out, L, Df, jb::EPI_BIAS)) return 1;   // first L rows of Wmv = fc_mus
+    if (addc(hB, hf, mf.Wmv, mf.bmv, out, ld_out, L, Df, jb::EPI_BIAS, 1, 0)) return 1;   // first L rows of Wmv = fc_mus
   } else {
     ModSegs& mt = e->ms[to];
     const int Dt = e->D[to];
-    const int ld2t = r4(2 * Dt), ldt = r4(Dt);
-    if (add(bufB, ldf, mf.Wmv, mf.bmv, 0, bufA, e->LP, L, Df, jb::EPI_BIAS)) return 1;
-    if (add(bufA, e->LP, mt.W3, mt.b3, 0, bufB, ldt, Dt, L, jb::EPI_BIAS_LRELU)) return 1;
-    if (add(bufB, ldt, mt.W4, mt.b4, 0, bufA, ld2t, 2 * Dt, Dt, jb::EPI_BIAS_LRELU)) return 1;
-    if (add(bufA, ld2t, mt.W5, mt.b5, 0, out, ld_out, Dt, 2 * Dt, jb::EPI_BIAS)) return 1;
+    const int h2t = r8(2 * Dt), ht = r8(Dt);
+    if (addc(hB, hf, mf.Wmv, mf.bmv, bufA, e->LP, L, Df, jb::EPI_BIAS, 1, 0)) return 1;
+    if (addc(bufA, e->LP, mt.W3, mt.b3, hB, ht, Dt, L, jb::EPI_BIAS_LRELU, 0, 1)) return 1;
+    if (addc(hB, ht, mt.W4, mt.b4, hA, h2t, 2 * Dt, Dt, jb::EPI_BIAS_LRELU, 1, 1)) return 1;
+    if (addc(hA, h2t, mt.W5, mt.b5, out, ld_out, Dt, 2 * Dt, jb::EPI_BIAS, 1, 0)) return 1;
   }
   CU(cudaMemcpyAsync(d_tab, tab.data(), tab.size() * sizeof(GemmProblem), cudaMemcpyHostToDevice, s));
   for (size_t k = 0; k < tab.size(); ++k) {
     // programmatic dependent launch inside the chain: GEMM k + 1 sets up while GEMM k drains (the kernel waits for its
     // predecessor before touching memory)
-    if (e->eval_persist) CU(jb::gemm_launch_persistent(d_tab + k, tab[k], e->num_sms, s, k > 0));
-    else CU(jb::gemm_launch(d_tab + k, 1, tab[k].tiles_m * tab[k].tiles_n, s, k > 0));
+    CU(jb::gemm_launch_persistent(d_tab + k, tab[k], e->num_sms, s, k > 0));
     ++e->launches;
   }
   return 0;
@@ -887,7 +831,6 @@ int jb_create(const jb_config* cfg, jb_engine** out) {
   if (!prop.cooperativeLaunch) return fail("the device does not support cooperative launches");
   jb_engine* e = new jb_engine();
   e->cfg = *cfg;
-  if (const char* pv = getenv("JB_PRECISION")) e->precision_fast = strcmp(pv, "f16") == 0 || strcmp(pv, "tf32") == 0;
   e->D[0] = cfg->dims[0]; e->D[1] = cfg->dims[1]; e->L = cfg->latent; e->LP = r8(cfg->latent); e->ldmv = r8(2 * cfg->latent);
   e->Bmax = cfg->max_batch;
   build_layout(e);
@@ -924,13 +867,8 @@ int jb_create(const jb_config* cfg, jb_engine** out) {
   e->norm_tile = nullptr; e->norm_tile_cap = 0;   // sized by build_step (one partial per epilogue warp and weight-gradient work item)
   CU(cudaMalloc(&e->norm_small, jb::SK_MAX_CTAS * 4 * sizeof(float)));
   CU(cudaMemset(e->norm_small, 0, jb::SK_MAX_CTAS * 4 * sizeof(float)));
-  if (const char* pv = getenv("JB_NORM_FUSE")) e->norm_fuse = atoi(pv) != 0;
   CU(cudaMalloc(&e->bar, 512));
   CU(cudaMemset(e->bar, 0, 512));
-  if (const char* pv = getenv("JB_WGRAD_BN")) e->wgrad_bn = atoi(pv);
-  if (const char* pv = getenv("JB_FWD_MODE")) e->fwd_mode = strcmp(pv, "medium") == 0 ? jb::HG_MEDIUM : (strcmp(pv, "precise") == 0 ? jb::HG_PRECISE : -1);
-  if (const char* pv = getenv("JB_WGRAD_MODE")) e->wgrad_mode = strcmp(pv, "single") == 0 ? jb::HG_SINGLE : jb::HG_MEDIUM;
-  if (const char* pv = getenv("JB_MAX_KSPLIT")) { if (atoi(pv) >= 1) e->max_ksplit = atoi(pv); }
   CU(cudaFuncSetAttribute(jb::gemm_tf32_grouped_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, jb::GEMM_SMEM_BYTES));
   CU(cudaFuncSetAttribute(jb::k_step, cudaFuncAttributeMaxDynamicSharedMemorySize, jb::HG_SMEM_BYTES));
   e->num_sms = prop.multiProcessorCount;
@@ -947,18 +885,10 @@ int jb_create(const jb_config* cfg, jb_engine** out) {
     if (nclusters < 1) { jb_destroy(e); return fail("the step kernel does not fit on the device (shared memory / registers / clusters)"); }
     e->grid = nclusters * jb::HG_CLUSTER;
     if (e->grid > jb::SK_MAX_CTAS) e->grid = (jb::SK_MAX_CTAS / jb::HG_CLUSTER) * jb::HG_CLUSTER;
-    if (const char* pv = getenv("JB_STEP_CTAS")) { const int v = atoi(pv) / jb::HG_CLUSTER * jb::HG_CLUSTER; if (v >= jb::HG_CLUSTER && v <= e->grid) e->grid = v; }
-    if (const char* pv = getenv("JB_FUSE")) e->fuse_enabled = atoi(pv) != 0;
-    if (const char* pv = getenv("JB_MERGE_LATENT")) e->merge_latent = atoi(pv) != 0;
-    if (const char* pv = getenv("JB_FUSE_KS")) e->fuse_ks = atoi(pv) != 0;
   }
   // rows per pass of the folded chain: one 128-row M tile per SM, so every GEMM of the chain is a whole number of waves
   // (measured on B200, 1M rows 512 -> 512: 8192 rows 59.1, 9472 rows 66.7, 18944 rows 69.0 M rows/s)
   e->eval_chunk = 128 * e->num_sms;
-  if (const char* pv = getenv("JB_EVAL_CHUNK")) { if (atoi(pv) >= 128) e->eval_chunk = atoi(pv); }
-  if (const char* pv = getenv("JB_EVAL_BN256_MIN")) e->eval_bn256_min = atoi(pv);
-  if (const char* pv = getenv("JB_EVAL_PERSIST")) e->eval_persist = atoi(pv) != 0;
-  if (const char* pv = getenv("JB_EVAL_F16")) e->eval_f16 = atoi(pv) != 0;
   CU(cudaMalloc(&e->theta_eval_h, static_cast<size_t>(e->n_flat + 32) * 2));
   // eval workspaces: two slots of chunk activations
   {

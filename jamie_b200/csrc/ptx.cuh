@@ -143,30 +143,9 @@ __device__ __forceinline__ void bulk_store(void* gdst, const void* smem_src, uin
                "r"(bytes)
                : "memory");
 }
-// the same with an L2 eviction policy (createpolicy): streams that are touched once per step should not displace the
-// operands the GEMM phases re-read
-__device__ __forceinline__ uint64_t l2_policy_evict_first() {
-  uint64_t p;
-  asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p));
-  return p;
-}
-__device__ __forceinline__ void bulk_load_hint(void* smem_dst, const void* gsrc, uint32_t bytes, uint64_t* bar, uint64_t policy) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1], %2, [%3], %4;" ::"r"(smem_u32(smem_dst)),
-               "l"(reinterpret_cast<uint64_t>(gsrc)), "r"(bytes), "r"(smem_u32(bar)), "l"(policy)
-               : "memory");
-}
-__device__ __forceinline__ void bulk_store_hint(void* gdst, const void* smem_src, uint32_t bytes, uint64_t policy) {
-  asm volatile("cp.async.bulk.global.shared::cta.bulk_group.L2::cache_hint [%0], [%1], %2, %3;" ::"l"(reinterpret_cast<uint64_t>(gdst)),
-               "r"(smem_u32(smem_src)), "r"(bytes), "l"(policy)
-               : "memory");
-}
 __device__ __forceinline__ void bulk_wait_read_1() { asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory"); }
 
 // ---------------------------------------------------------------- L2 prefetch
-// Bulk prefetch of `bytes` (a multiple of 16, 16-byte aligned) of global memory into L2: one instruction, no destination.
-__device__ __forceinline__ void prefetch_l2_bulk(const void* p, uint32_t bytes) {
-  asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(reinterpret_cast<uint64_t>(p)), "r"(bytes) : "memory");
-}
 // TMA prefetch of one tensor-map box into L2 (no shared-memory destination, no barrier)
 __device__ __forceinline__ void tma_prefetch_2d(const void* tmap, int c0, int c1) {
   asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global.tile [%0, {%1, %2}];" ::"l"(reinterpret_cast<uint64_t>(tmap)), "r"(c0), "r"(c1) : "memory");

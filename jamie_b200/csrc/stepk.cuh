@@ -130,13 +130,12 @@ struct StepCtx {
   // BatchNorm affine, sigma: norm_rng (offset, length) pairs) are summed by warps without a GEMM role during WGRAD into
   // norm_small [4 ncta]
   float *norm_tile, *norm_small;
-  int n_norm_tile, n_norm_rng, norm_fuse;
+  int n_norm_tile, n_norm_rng;
   int norm_rng[32][2];
   // plan / control / outputs
   const float* plan_kl; float* out_loss; Ctl* ctl;
   StepConsts sc;
   float gs, inv_gs;                // loss scale of the backward pass and its inverse
-  int dbg_repeat;                  // 1
   int merge_latent;                // no F: LATLOSS / LATFIN folded into COMBINE / LATBZ / the DEC1 and DGH phases (optimistic operand scales)
   int eps_early;                   // the reparameterisation noise is drawn during ENC1 (heads tail fused)
   // in-kernel data-parallel exchange (sk_exchange); xworld <= 1: off
@@ -144,8 +143,6 @@ struct StepCtx {
   int xfence;                      // 1: every exchange fence at system scope (JB_XCHG_FENCE=sys); 0: see fence_light
   long long x_adam0;               // optimizer step count when the exchange was configured (epoch 0 of the flags)
   float* xmc;                      // NVSwitch multicast address of the gradient buffers (NULL: peer loads / stores)
-  int adam_stream;                 // JB_ADAM_STREAM=0: plain-load Adam sweep
-  int prefetch_state;              // JB_PREFETCH_STATE=1 (default 0, measured slower): L2 prefetch of theta, m, v during WGRAD
   unsigned long long phase_mask;   // bit ph set: the phase runs (fused layers drop the BatchNorm / REC / REPARAM phases)
   // GEMM tables
   HgPhase gph[SK_NUM_GEMM];
@@ -1734,7 +1731,6 @@ __device__ __forceinline__ void sk_adam_stream(const StepCtx& cx, uint8_t* ring,
   // bars[0 .. STAGES) are initialised once per launch (k_step prologue); bars[STAGES] holds their parity bits between
   // uses (an initialised mbarrier must not be initialised again)
   uint32_t par = *reinterpret_cast<volatile uint32_t*>(&bars[ADAM_STAGES]);
-  const uint64_t pol = l2_policy_evict_first();
   __syncthreads();
   auto issue = [&](int k) {   // thread 0: loads of this CTA's k-th chunk
     const long long c = cta + static_cast<long long>(k) * ncta;
@@ -1744,17 +1740,10 @@ __device__ __forceinline__ void sk_adam_stream(const StepCtx& cx, uint8_t* ring,
     uint8_t* st = ring + (k % ADAM_STAGES) * ADAM_STAGE_BYTES;
     uint64_t* bar = &bars[k % ADAM_STAGES];
     mbar_arrive_expect_tx(bar, 4 * bytes);
-    if (cx.adam_stream == 2) {
-      bulk_load_hint(st, cx.grad + e0, bytes, bar, pol);
-      bulk_load_hint(st + ADAM_CHUNK * 4, cx.adam_m + e0, bytes, bar, pol);
-      bulk_load_hint(st + 2 * ADAM_CHUNK * 4, cx.adam_v + e0, bytes, bar, pol);
-      bulk_load_hint(st + 3 * ADAM_CHUNK * 4, cx.theta + e0, bytes, bar, pol);
-    } else {
-      bulk_load(st, cx.grad + e0, bytes, bar);
-      bulk_load(st + ADAM_CHUNK * 4, cx.adam_m + e0, bytes, bar);
-      bulk_load(st + 2 * ADAM_CHUNK * 4, cx.adam_v + e0, bytes, bar);
-      bulk_load(st + 3 * ADAM_CHUNK * 4, cx.theta + e0, bytes, bar);
-    }
+    bulk_load(st, cx.grad + e0, bytes, bar);
+    bulk_load(st + ADAM_CHUNK * 4, cx.adam_m + e0, bytes, bar);
+    bulk_load(st + 2 * ADAM_CHUNK * 4, cx.adam_v + e0, bytes, bar);
+    bulk_load(st + 3 * ADAM_CHUNK * 4, cx.theta + e0, bytes, bar);
   };
   if (tid == 0)
     for (int k = 0; k < ADAM_STAGES - 2 && k < mine; ++k) issue(k);
@@ -1799,15 +1788,9 @@ __device__ __forceinline__ void sk_adam_stream(const StepCtx& cx, uint8_t* ring,
     __syncthreads();
     if (tid == 0) {
       const uint32_t bytes = static_cast<uint32_t>(n) * 4;
-      if (cx.adam_stream == 2) {
-        bulk_store_hint(cx.adam_m + e0, st + ADAM_CHUNK * 4, bytes, pol);
-        bulk_store_hint(cx.adam_v + e0, st + 2 * ADAM_CHUNK * 4, bytes, pol);
-        bulk_store_hint(cx.theta + e0, st + 3 * ADAM_CHUNK * 4, bytes, pol);
-      } else {
-        bulk_store(cx.adam_m + e0, st + ADAM_CHUNK * 4, bytes);
-        bulk_store(cx.adam_v + e0, st + 2 * ADAM_CHUNK * 4, bytes);
-        bulk_store(cx.theta + e0, st + 3 * ADAM_CHUNK * 4, bytes);
-      }
+      bulk_store(cx.adam_m + e0, st + ADAM_CHUNK * 4, bytes);
+      bulk_store(cx.adam_v + e0, st + 2 * ADAM_CHUNK * 4, bytes);
+      bulk_store(cx.theta + e0, st + 3 * ADAM_CHUNK * 4, bytes);
       bulk_store(cx.theta_hi + e0, st, bytes / 2);
       bulk_store(cx.theta_lo + e0, st + ADAM_CHUNK * 2, bytes / 2);
       tma_store_commit();
@@ -1822,6 +1805,8 @@ __device__ __forceinline__ void sk_adam_stream(const StepCtx& cx, uint8_t* ring,
 }
 // every CTA re-reduces the partials in the same order (identical clip coefficient everywhere), then
 // g *= grad_scale * clip;  m, v, theta updated with torch.optim.Adam's formulas (jamie/jamie.py:739-741).
+// theta, m, v are not prefetched into L2 during WGRAD: measured on B200, a bulk L2 prefetch by the warps without a GEMM
+// role took 3.5 us off ADAM but added 9.4 us to WGRAD (it competes with the operand loads).
 __device__ __forceinline__ void sk_adam(const StepCtx& cx, const StepVars& sv, int cta, int ncta, double* shd, int tid, bool fused_norm, uint8_t* ring, uint64_t* abars) {
   double s = 0.0;
   if (cx.xworld > 1) {   // partial sums of squares of the reduced slices, delivered by every rank (sk_exchange)
@@ -1847,48 +1832,7 @@ __device__ __forceinline__ void sk_adam(const StepCtx& cx, const StepVars& sv, i
   __syncthreads();
   const float b1 = sc.beta1, b2 = sc.beta2, eps = sc.adam_eps;
   const float step = sv.step_size, ibc2 = sv.inv_bc2_sqrt;
-  if (cx.adam_stream) {
-    sk_adam_stream(cx, ring, abars, cta, ncta, tid, coef, b1, b2, eps, step, ibc2);
-    return;
-  }
-  const long long n4 = cx.n_flat / 4;
-  float4* t4 = reinterpret_cast<float4*>(cx.theta);
-  const float4* g4 = reinterpret_cast<const float4*>(cx.grad);
-  float4* m4 = reinterpret_cast<float4*>(cx.adam_m);
-  float4* v4 = reinterpret_cast<float4*>(cx.adam_v);
-  const long long stride = static_cast<long long>(ncta) * SK_THREADS;
-  // The sweep: 8 independent 16-byte loads per thread before the first use. Measured alternatives (B200): 16 loads in
-  // flight (U = 4) spills inside the 128-register budget and takes 45.8 us instead of 31; theta / m / v prefetched into L2
-  // during WGRAD (JB_PREFETCH_STATE=1) brings the phase to 27.6 us but costs WGRAD 9.4 us: the phase moves 121 MB at
-  // 3.9 TB/s = 60 % of the measured copy bandwidth with nine interleaved streams.
-#pragma unroll 1
-  for (long long i0 = static_cast<long long>(cta) * SK_THREADS + tid; i0 < n4; i0 += 2 * stride) {   // 8 loads in flight
-    float4 gg[2], mm[2], vv[2], tt[2];
-#pragma unroll
-    for (int u = 0; u < 2; ++u) {
-      const long long i = i0 + u * stride < n4 ? i0 + u * stride : n4 - 1;   // clamped, not predicated: every register is defined
-      gg[u] = sk_ld(g4 + i); mm[u] = m4[i]; vv[u] = v4[i]; tt[u] = t4[i];
-    }
-#pragma unroll
-    for (int u = 0; u < 2; ++u) {
-      const long long i = i0 + u * stride;
-      if (i < n4) {
-        const float gx[4] = {gg[u].x * coef, gg[u].y * coef, gg[u].z * coef, gg[u].w * coef};
-        float* mp = reinterpret_cast<float*>(&mm[u]);
-        float* vp = reinterpret_cast<float*>(&vv[u]);
-        float* tp = reinterpret_cast<float*>(&tt[u]);
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-          mp[k] = mp[k] + (gx[k] - mp[k]) * (1.f - b1);
-          vp[k] = vp[k] * b2 + gx[k] * gx[k] * (1.f - b2);
-          const float denom = sqrtf(vp[k]) * ibc2 + eps;
-          tp[k] = tp[k] - step * (mp[k] / denom);
-        }
-        m4[i] = mm[u]; v4[i] = vv[u]; t4[i] = tt[u];
-        split4_store(cx.theta_hi + 4 * i, cx.theta_lo + 4 * i, tt[u].x, tt[u].y, tt[u].z, tt[u].w);   // next step's GEMM operand planes
-      }
-    }
-  }
+  sk_adam_stream(cx, ring, abars, cta, ncta, tid, coef, b1, b2, eps, step, ibc2);
 }
 
 // sum of squares of the gradients of the small tensors (everything that is not a weight matrix): 128 threads per CTA
@@ -1927,21 +1871,6 @@ __device__ __forceinline__ void sk_running_stats(const StepCtx& cx, int gt, int 
       Lr.run_mean[c] = (1.f - BN_MOM) * Lr.run_mean[c] + BN_MOM * m;
       Lr.run_var[c] = (1.f - BN_MOM) * Lr.run_var[c] + BN_MOM * v * ub;
     }
-  }
-}
-
-// theta, m, v (52 MB at the headline shape) are pulled into L2 while the WGRAD GEMMs run, by the warps without a GEMM
-// role: the ADAM phase that follows (after NORM) then reads L2 instead of HBM. 16 KB per instruction.
-__device__ __forceinline__ void sk_prefetch_state(const StepCtx& cx, int gt, int nt) {
-  const long long bytes = cx.n_flat * 4;
-  const long long nchunk = (bytes + 16383) >> 14;
-#pragma unroll 1
-  for (long long i = gt; i < 3 * nchunk; i += nt) {
-    const int which = static_cast<int>(i / nchunk);
-    const long long off = (i - which * nchunk) << 14;
-    const char* base = reinterpret_cast<const char*>(which == 0 ? cx.theta : (which == 1 ? cx.adam_m : cx.adam_v));
-    const long long left = bytes - off;
-    prefetch_l2_bulk(base + off, static_cast<uint32_t>(left < 16384 ? left : 16384));
   }
 }
 
@@ -2003,13 +1932,13 @@ __global__ void __launch_bounds__(SK_THREADS, 1) k_step(const __grid_constant__ 
   unsigned int target = 0;
   if (cta == 0 && tid == 0) *bar_next = 0u;
   const int B = cx.B;
-  const bool norm_fused = cx.norm_fuse != 0 && ph_lo <= PH_DG3 && ph_hi > PH_ADAM && cx.xworld <= 1;   // every weight-gradient epilogue of the step is in this launch
   // the counters CTA 0 advances at the end are read once, before this CTA's first grid barrier (used by thread 0 only)
   long long ctl_cursor0 = 0, ctl_adam0 = 0;
   unsigned long long ctl_stream0 = 0;
   if (tid == 0) { ctl_cursor0 = cx.ctl->cursor; ctl_adam0 = cx.ctl->adam_t; ctl_stream0 = cx.ctl->stream_id; }
   const long long ctl_xepoch = cx.xworld > 1 ? cx.ctl->adam_t - cx.x_adam0 : 0;   // exchange epochs = optimizer steps: the same on every rank
 
+  const bool norm_fused = ph_lo <= PH_DG3 && ph_hi > PH_ADAM && cx.xworld <= 1;   // every weight-gradient epilogue of the step is in this launch
   if (ts != nullptr && cta == 0 && tid == 0) ts[0] = globaltimer_ns();
   long long clk_begin = clock64();
   for (int s = 0; s < nsteps; ++s) {
@@ -2054,7 +1983,6 @@ __global__ void __launch_bounds__(SK_THREADS, 1) k_step(const __grid_constant__ 
         }
         const HgPhase& gphase = cx.gph[gi];
         if (ph == PH_WGRAD && warp >= HG_WARP_EPI0 + HG_NEPI) {
-          if (cx.prefetch_state && ph_hi > PH_ADAM) sk_prefetch_state(cx, cta * 128 + (tid - 32 * (HG_WARP_EPI0 + HG_NEPI)), ncta * 128);
           if (!((cx.phase_mask >> PH_BN1) & 1ull)) sk_running_stats(cx, cta * 128 + (tid - 32 * (HG_WARP_EPI0 + HG_NEPI)), ncta * 128);
           if (norm_fused) sk_norm_small(cx, cta, ncta, warp - (HG_WARP_EPI0 + HG_NEPI), lane);
         }
@@ -2083,7 +2011,6 @@ __global__ void __launch_bounds__(SK_THREADS, 1) k_step(const __grid_constant__ 
             if (tid == 0) ta.stamp[7] = clk_begin;
           }
           const int arg = P.fuse_arg;
-          for (int rep = 0; rep < cx.dbg_repeat; ++rep)
           switch (P.fuse) {
             case FUSE_BN_FWD: sk_tail_bn_fwd(cx, sv, cx.bn[arg >> 1][arg & 1], P.bias, ta); break;
             case FUSE_BN_BWD: sk_tail_bn_bwd(cx, sv, cx.bn[arg >> 1][arg & 1], ta); break;
@@ -2117,7 +2044,6 @@ __global__ void __launch_bounds__(SK_THREADS, 1) k_step(const __grid_constant__ 
             if ((ncta - 1 - (it % ncta)) == cta) { __syncthreads(); sk_final_item(cx, sv, it, sh, tid, warp, lane); }
         }
       } else {
-       for (int rep = 0; rep < cx.dbg_repeat; ++rep) {   // timing experiments only (JB_DBG_REPEAT): repeats the phase's work
         switch (ph) {
           case PH_GATHER: {
             // warp items: B rows of the P / F blocks (from the top of the grid down), then 2 B batch rows
@@ -2196,7 +2122,6 @@ __global__ void __launch_bounds__(SK_THREADS, 1) k_step(const __grid_constant__ 
           case PH_ADAM: sk_adam(cx, sv, cta, ncta, shd, tid, norm_fused, ring, reinterpret_cast<uint64_t*>(smem + 192)); break;
           default: break;
         }
-       }
       }
       const bool last = (ph == ph_hi - 1) && (s == nsteps - 1);
       if (ts != nullptr) {   // per-CTA detail: SM clock at the end of this CTA's work, global time at that moment

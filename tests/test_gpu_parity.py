@@ -108,6 +108,7 @@ SHAPES = [
     ([2000, 1000], 32, 300, 0.6, 'eye', False),     # MMD-MA without PCA (config 1)
     ([96, 64], 8, 64, 0.0, 'zeros', True),          # no dropout, zero prior, dense F with PF_Ratio < 1
     ([130, 70], 17, 50, 0.3, 'dense', True),        # odd everything: widths, latent, batch
+    ([96, 64], 8, 640, 0.3, 'eye', False),          # B > 512: the unfused BatchNorm / reconstruction / reparam phases
 ]
 
 

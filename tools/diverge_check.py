@@ -1,5 +1,5 @@
 """Where does a long run of the bench workload leave the finite range? Prints the loss trajectory and the first
-non-finite step for the forward-GEMM modes (JB_FWD_MODE) on the bench's own data, plan and seeds (N = 1)."""
+non-finite step on the bench's own data, plan and seeds (N = 1)."""
 import os, sys
 import numpy as np
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), '..'))
@@ -13,8 +13,7 @@ torch.cuda.set_device(0)
 g = torch.Generator(device='cuda').manual_seed(1234)
 data = [torch.randn((n, d), generator=g, device='cuda', dtype=torch.float32) for d in Bn.DIMS]
 SEEDS = [int(x) for x in os.environ.get('JB_DIV_SEEDS', '0').split(',')]
-for mode, seed in [(m, sd) for m in (sys.argv[3:] or ['auto', 'precise']) for sd in SEEDS]:
-    os.environ['JB_FWD_MODE'] = mode
+for seed in SEEDS:
     rng = np.random.default_rng(100 + seed)
     mask = (rng.random(n) < 0.5).astype(np.float32)
     nz = np.flatnonzero(mask)[:2]
@@ -31,7 +30,7 @@ for mode, seed in [(m, sd) for m in (sys.argv[3:] or ['auto', 'precise']) for sd
     torch.cuda.synchronize()
     ls = eng.read_losses(steps)
     bad = np.flatnonzero(~np.isfinite(ls[:, :6]).all(axis=1))
-    print(f'JB_FWD_MODE={mode} seed {seed}: max total loss {np.nanmax(ls[:, 4]):.3g} at step {int(np.nanargmax(ls[:, 4]))}, max |g| {np.nanmax(ls[:, 5]):.3g}; first non-finite step: {int(bad[0]) if bad.size else None} of {steps}')
+    print(f'seed {seed}: max total loss {np.nanmax(ls[:, 4]):.3g} at step {int(np.nanargmax(ls[:, 4]))}, max |g| {np.nanmax(ls[:, 5]):.3g}; first non-finite step: {int(bad[0]) if bad.size else None} of {steps}')
     for s in (list(range(0, steps, max(steps // 16, 1))) if os.environ.get('JB_DIV_VERBOSE') else []) + ([int(bad[0]) - 2, int(bad[0]) - 1, int(bad[0])] if bad.size else []):
         if 0 <= s < steps:
             print(f'  step {s:5d}: KL {ls[s, 0]:.4g} Rec {ls[s, 1]:.4g} Cos {ls[s, 2]:.4g} F {ls[s, 3]:.4g} total {ls[s, 4]:.4g} |g| {ls[s, 5]:.4g}')
