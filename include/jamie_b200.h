@@ -187,6 +187,27 @@ int jb_pca_project(jb_engine* e, const float* X, long long n, long long d, const
 int jb_pca_inverse(jb_engine* e, const float* Z, long long n, int k, const float* comp, const float* mean,
                    long long d, float m, float s, float* out, int on_device, void* stream);
 
+/* Feature ablation (SURVEY.md 3.2: the notebooks' loops that replace one raw input feature, rerun modal_predict or
+ * transform_one and score the result, once per feature; jamie_b200/impact.py). For every ablated feature j the network's
+ * input is Z(j) = Z + dz[j] w_j^T, a rank-1 update of the unablated input Z = preprocessing[from](X):
+ *   Z     [n, dims[from]] float64 host.   dz [n_feat][n] float64 host: f_j - X[:, j] per feature.
+ *   w     w_col == NULL: [n_feat, dims[from]] (components_[:, j] / s of a PCA input side);
+ *         else [n_feat] scalars added to column w_col[j] only (1 / s_j of a side standardised per column).
+ * Y(j) = map(chain(Z(j))), chain = encoder -> mu (to = -1) or encoder -> mu -> decoder[to], in eval mode as jb_encode /
+ * jb_predict; map_kind 0 = identity (d_out = the chain's width), 1 = the PCA inverse of jb_pca_inverse (comp [D_to, d_out],
+ * mean [d_out], scalar m / s), 2 = fp32(y * aff_scale[c] + aff_shift[c]) (d_out = D_to). Y(-) is Y of the unablated Z.
+ *   shift [n_feat, d_out] : mean over rows of |Y(j)[:, c] - Y(-)[:, c]|
+ *   with target [n, d_out] fp32 (else NULL): base_r [d_out] = Pearson r(Y(-)[:, c], target[:, c]) and r [n_feat, d_out] the
+ *   same for Y(j), finished as jb_metric_feature_pearson does (a constant column gives nan).
+ * Works in batches of features x row ranges whose working set stays under batch_bytes (and the free memory): no
+ * prediction leaves the device. Sums are float64 per 32-row slab at fixed absolute rows, folded in row order: results are
+ * bit-identical across reruns and for any batch_bytes. Refuses, before any allocation, a problem whose smallest batch
+ * (one feature, 32 rows) does not fit in free device memory. Host pointers; synchronous. */
+int jb_feature_impact(jb_engine* e, int from, int to, const double* Z, long long n, long long n_feat, const double* dz,
+                      const double* w, const int* w_col, int map_kind, const float* comp, const float* mean, float m, float s,
+                      const double* aff_scale, const double* aff_shift, long long d_out, const float* target, double* base_r,
+                      double* r, double* shift, long long batch_bytes, void* stream);
+
 /* PCA fit (jamie/jamie.py:436-452, sklearn PCA(n_components).fit with the covariance_eigh solver): the two O(n d) /
  * O(n d^2) passes over the [n, d] matrix run on the GPU -- column sums, then the centred Gram matrix
  * (X - mean)^T (X - mean) as a split (fp32-class) tensor-core GEMM accumulated over row chunks in float64. The caller

@@ -35,6 +35,7 @@
 #include "metrics.cuh"
 #include "distances.cuh"
 #include "pcaop.cuh"
+#include "impact.cuh"
 
 namespace {
 
@@ -1614,22 +1615,51 @@ int jb_pca_gram(jb_engine* e, const float* X, long long n, long long d, const do
   return 0;
 }
 
+namespace {
+// preclass.inverse_transform with PCA on device rows: out = (Z * s + m) @ comp + mean. The component hi/lo planes are split
+// once (prepare); apply then maps any number of row blocks (jb_pca_inverse's chunks, jb_feature_impact's batches).
+struct PcaInverse {
+  DevBuf c_raw, c_hi, c_lo, d_mean;
+  int k = 0, ldk = 0;
+  long long d = 0, ldd = 0;
+  float m = 0.f, s = 1.f;
+  int prepare(jb_engine* e, const float* comp, const float* mean, int k_, long long d_, float m_, float s_, cudaStream_t st) {
+    k = k_; d = d_; m = m_; s = s_;
+    ldd = r4(static_cast<int>(d));
+    ldk = r4(k);
+    if (c_raw.alloc(static_cast<size_t>(k) * d) || c_hi.alloc(static_cast<size_t>(k) * ldd) ||
+        c_lo.alloc(static_cast<size_t>(k) * ldd) || d_mean.alloc(d)) return 1;
+    CU(cudaMemcpyAsync(c_raw.p, comp, static_cast<size_t>(k) * d * 4, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(d_mean.p, mean, static_cast<size_t>(d) * 4, cudaMemcpyHostToDevice, st));
+    jb::k_split_tf32<<<k, 256, 0, st>>>(c_raw.p, d, k, static_cast<int>(d), 2, nullptr, 1.f, 0.f, c_hi.p, c_lo.p, ldd); ++e->launches;
+    return 0;
+  }
+  // Z: [rows, ldz] device; z_hi / z_lo: [rows, ldk] scratch; out: [rows, ldd] device
+  int apply(jb_engine* e, const float* Z, long long ldz, long long rows, float* z_hi, float* z_lo, float* out, cudaStream_t st) {
+    jb::k_split_tf32<<<static_cast<unsigned>(rows), 128, 0, st>>>(Z, ldz, rows, k, 1, nullptr, s, m, z_hi, z_lo, ldk); ++e->launches;
+    GemmProblem g;   // out[rows, d] = A[rows, k] * comp[k, d]: B is logically [N = d, K = k] stored [k][d] -> MN-major
+    int rc = jb::gemm_problem_fill(&g, z_hi, ldk, 0, c_hi.p, static_cast<int>(ldd), 1, out, static_cast<int>(ldd),
+                                   static_cast<int>(rows), static_cast<int>(d), k, 64, jb::EPI_BIAS, d_mean.p, 0.f, 0, 0,
+                                   z_lo, c_lo.p);
+    if (rc) return fail("PCA tensor map encode failed (%d)", rc);
+    return launch_one(e, g, e->d_ev_probs, st);
+  }
+};
+}  // namespace
+
 int jb_pca_inverse(jb_engine* e, const float* Z, long long n, int k, const float* comp, const float* mean, long long d,
                    float m, float sdev, float* out, int on_device, void* stream) {
   if (!e || !Z || !comp || !mean || !out) return fail("null argument");
   if (n <= 0 || d <= 0 || k <= 0) return fail("bad PCA shape");
   cudaStream_t s = static_cast<cudaStream_t>(stream);
-  const long long ldd = r4(static_cast<int>(d));
-  const int ldk = r4(k);
+  PcaInverse inv;
+  if (inv.prepare(e, comp, mean, k, d, m, sdev, s)) return 1;
+  const long long ldd = inv.ldd;
   const long long R = pca_chunk_rows(ldd);
-  DevBuf c_raw, c_hi, c_lo, d_mean, z_raw, z_hi, z_lo, o;
-  if (c_raw.alloc(static_cast<size_t>(k) * d) || c_hi.alloc(static_cast<size_t>(k) * ldd) || c_lo.alloc(static_cast<size_t>(k) * ldd) ||
-      d_mean.alloc(d) || z_hi.alloc(static_cast<size_t>(R) * ldk) || z_lo.alloc(static_cast<size_t>(R) * ldk) ||
+  DevBuf z_raw, z_hi, z_lo, o;
+  if (z_hi.alloc(static_cast<size_t>(R) * inv.ldk) || z_lo.alloc(static_cast<size_t>(R) * inv.ldk) ||
       o.alloc(static_cast<size_t>(R) * ldd)) return 1;
   if (!on_device && z_raw.alloc(static_cast<size_t>(R) * k)) return 1;
-  CU(cudaMemcpyAsync(c_raw.p, comp, static_cast<size_t>(k) * d * 4, cudaMemcpyHostToDevice, s));
-  CU(cudaMemcpyAsync(d_mean.p, mean, static_cast<size_t>(d) * 4, cudaMemcpyHostToDevice, s));
-  jb::k_split_tf32<<<k, 256, 0, s>>>(c_raw.p, d, k, static_cast<int>(d), 2, nullptr, 1.f, 0.f, c_hi.p, c_lo.p, ldd); ++e->launches;
   for (long long r0 = 0; r0 < n; r0 += R) {
     const long long rows = n - r0 < R ? n - r0 : R;
     const float* src = Z + r0 * k;
@@ -1637,20 +1667,129 @@ int jb_pca_inverse(jb_engine* e, const float* Z, long long n, int k, const float
       CU(cudaMemcpyAsync(z_raw.p, src, static_cast<size_t>(rows) * k * 4, cudaMemcpyHostToDevice, s));
       src = z_raw.p;
     }
-    jb::k_split_tf32<<<static_cast<unsigned>(rows), 128, 0, s>>>(src, k, rows, k, 1, nullptr, sdev, m, z_hi.p, z_lo.p, ldk); ++e->launches;
-    {
-      GemmProblem g;   // out[rows, d] = A[rows, k] * comp[k, d]: B is logically [N = d, K = k] stored [k][d] -> MN-major
-      int rc = jb::gemm_problem_fill(&g, z_hi.p, ldk, 0, c_hi.p, static_cast<int>(ldd), 1, o.p, static_cast<int>(ldd),
-                                     static_cast<int>(rows), static_cast<int>(d), k, 64, jb::EPI_BIAS, d_mean.p, 0.f, 0, 0,
-                                     z_lo.p, c_lo.p);
-      if (rc) return fail("PCA tensor map encode failed (%d)", rc);
-      if (launch_one(e, g, e->d_ev_probs, s)) return 1;
-    }
+    if (inv.apply(e, src, k, rows, z_hi.p, z_lo.p, o.p, s)) return 1;
     CU(cudaMemcpy2DAsync(out + r0 * d, static_cast<size_t>(d) * 4, o.p, static_cast<size_t>(ldd) * 4, static_cast<size_t>(d) * 4,
                          rows, on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, s));
     CU(cudaStreamSynchronize(s));
   }
   CU(cudaGetLastError());
+  return 0;
+}
+
+// ---------------------------------------------------------------------------------------------- feature ablation (SURVEY 3.2)
+
+int jb_feature_impact(jb_engine* e, int from, int to, const double* Z, long long n, long long n_feat, const double* dz,
+                      const double* w, const int* w_col, int map_kind, const float* comp, const float* mean, float m, float sdev,
+                      const double* aff_scale, const double* aff_shift, long long d_out, const float* target, double* base_r,
+                      double* r, double* shift, long long batch_bytes, void* stream) {
+  if (!e || !Z || (n_feat > 0 && (!dz || !w || !shift))) return fail("null argument");
+  if (from < 0 || from > 1 || to < -1 || to > 1) return fail("modality index out of range");
+  if (n <= 0 || n_feat < 0 || d_out <= 0) return fail("bad feature-impact shape");
+  const int D_in = e->D[from];
+  const int D_to = to < 0 ? e->L : e->D[to];
+  if (map_kind == 1) {
+    if (!comp || !mean || to < 0) return fail("the PCA output map needs comp, mean and an output modality");
+  } else if (map_kind == 2) {
+    if (!aff_scale || !aff_shift || d_out != D_to) return fail("the per-column output map needs %d scales and shifts", D_to);
+  } else if (map_kind != 0 || d_out != D_to) {
+    return fail("output map %d with %lld output columns (the network gives %d)", map_kind, d_out, D_to);
+  }
+  if (target && (!base_r || !r)) return fail("a target needs base_r and r");
+  if (d_out > (1LL << 30) || n > (1LL << 40)) return fail("bad feature-impact shape");
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const long long SL = jb::IMP_SLAB;
+  const long long ldin = r4(D_in), ldto = r4(D_to), ldo = map_kind == 1 ? r4(static_cast<int>(d_out)) : ldto;
+  // bytes per row of one slot (ablated input, chain output, and for PCA the split planes and the inverse's output), per slot
+  // (its moment sums) and per feature (its dz column over all rows)
+  const double row_b = 4.0 * (ldin + ldto + (map_kind == 1 ? 2.0 * ldto + ldo : 0.0));
+  const double slot_b = 32.0 * d_out, feat_b = 8.0 * n;
+  const double fixed = 8.0 * n * D_in + (w_col ? 12.0 * n_feat : 8.0 * n_feat * D_in) + (target ? 4.0 * n * d_out : 0.0) +
+                       (map_kind == 1 ? 12.0 * D_to * ldo + 4.0 * d_out : 0.0) + (map_kind == 2 ? 16.0 * d_out : 0.0) + 16.0 * d_out;
+  auto batch = [&](long long a, long long R) { return (a + 1) * (R * row_b + slot_b) + a * feat_b; };
+  const long long n_pad = (n + SL - 1) / SL * SL;
+  const long long a_min = n_feat > 0 ? 1 : 0;
+  size_t free_b = 0, total_b = 0;
+  CU(cudaMemGetInfo(&free_b, &total_b));
+  const double avail = static_cast<double>(free_b) - (256.0 * (1 << 20));   // GEMM tables, tensor maps, allocator slack
+  const double need_min = fixed + batch(a_min, n_pad < SL ? n_pad : SL);
+  if (need_min > avail)
+    return fail("feature impact needs %.2f GB of device memory for its smallest batch (one feature, %lld rows); %.2f GB free",
+                need_min / 1e9, SL < n_pad ? SL : n_pad, static_cast<double>(free_b) / 1e9);
+  // row range: up to 1024 rows, halved while two slots of it exceed the budget; then as many features as fit
+  const double budget = static_cast<double>(batch_bytes) < avail - fixed ? static_cast<double>(batch_bytes) : avail - fixed;
+  long long R = n_pad < 1024 ? n_pad : 1024;
+  while (R > SL && batch(a_min, R) > budget) R = (R / 2 + SL - 1) / SL * SL;
+  long long a = a_min;
+  if (n_feat > 0) {
+    a = static_cast<long long>((budget - (R * row_b + slot_b)) / (R * row_b + slot_b + feat_b));
+    if (a < 1) a = 1;
+    if (a > n_feat) a = n_feat;
+    if (a > 65534) a = 65534;
+    while (a > 1 && fixed + batch(a, R) > avail) a /= 2;
+  }
+  const long long S = a + 1;
+  if ((S * R) > (1LL << 31) - 1) return fail("feature-impact batch of %lld rows", S * R);
+  if (prepare_eval(e, s)) return 1;
+
+  DevArr<double> dZ, dW, dDz, dAcc, dTacc, dSc, dSh;
+  DevArr<int> dWc;
+  DevArr<float> dT;
+  DevBuf xin, cout, zhi, zlo, o;
+  PcaInverse inv;
+  if (dZ.upload(Z, static_cast<size_t>(n) * D_in) || dAcc.alloc(static_cast<size_t>(S) * d_out * 4) ||
+      dTacc.alloc(static_cast<size_t>(2) * d_out) || xin.alloc(static_cast<size_t>(S * R) * ldin) ||
+      cout.alloc(static_cast<size_t>(S * R) * ldto)) return 1;
+  if (n_feat > 0) {
+    if (w_col ? (dW.upload(w, n_feat) || dWc.upload(w_col, n_feat)) : dW.upload(w, static_cast<size_t>(n_feat) * D_in)) return 1;
+    if (dDz.alloc(static_cast<size_t>(a) * n)) return 1;
+  }
+  if (target && dT.upload(target, static_cast<size_t>(n) * d_out)) return 1;
+  if (map_kind == 2 && (dSc.upload(aff_scale, d_out) || dSh.upload(aff_shift, d_out))) return 1;
+  if (map_kind == 1) {
+    if (inv.prepare(e, comp, mean, D_to, d_out, m, sdev, s) || zhi.alloc(static_cast<size_t>(S * R) * inv.ldk) ||
+        zlo.alloc(static_cast<size_t>(S * R) * inv.ldk) || o.alloc(static_cast<size_t>(S * R) * ldo)) return 1;
+  }
+  CU(cudaMemsetAsync(dTacc.p, 0, static_cast<size_t>(2) * d_out * sizeof(double), s));
+  std::vector<double> acc(static_cast<size_t>(S) * d_out * 4), tacc(static_cast<size_t>(2) * d_out);
+  const double N = static_cast<double>(n);
+  const unsigned mgrid = static_cast<unsigned>((d_out + 127) / 128);
+  for (long long j0 = 0; j0 < (n_feat > 0 ? n_feat : 1); j0 += (a > 0 ? a : 1)) {
+    const long long na = n_feat - j0 < a ? n_feat - j0 : a;   // features of this batch (slots 1 .. na)
+    if (na > 0) CU(cudaMemcpyAsync(dDz.p, dz + j0 * n, static_cast<size_t>(na) * n * 8, cudaMemcpyHostToDevice, s));
+    CU(cudaMemsetAsync(dAcc.p, 0, static_cast<size_t>(na + 1) * d_out * 4 * sizeof(double), s));
+    for (long long r0 = 0; r0 < n; r0 += R) {
+      const int rows = static_cast<int>(n - r0 < R ? n - r0 : R);
+      const long long brows = (na + 1) * rows;
+      jb::k_ablate_rows<<<static_cast<unsigned>(brows), 128, 0, s>>>(dZ.p, D_in, n, r0, rows, static_cast<int>(j0), dDz.p,
+                                                                     dW.p, dWc.p, xin.p, ldin); ++e->launches;
+      if (eval_common(e, from, to, xin.p, brows, ldin, cout.p, ldto, 1, s)) return 1;
+      const float* P = cout.p;
+      if (map_kind == 1) {
+        if (inv.apply(e, cout.p, ldto, brows, zhi.p, zlo.p, o.p, s)) return 1;
+        P = o.p;
+      }
+      jb::k_impact_moments<<<dim3(mgrid, static_cast<unsigned>(na + 1)), 128, 0, s>>>(
+          P, ldo, rows, r0, static_cast<int>(d_out), dT.p, dSc.p, dSh.p, dAcc.p, j0 == 0 ? dTacc.p : nullptr); ++e->launches;
+    }
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(acc.data(), dAcc.p, static_cast<size_t>(na + 1) * d_out * 4 * sizeof(double), cudaMemcpyDeviceToHost, s));
+    if (j0 == 0) CU(cudaMemcpyAsync(tacc.data(), dTacc.p, tacc.size() * sizeof(double), cudaMemcpyDeviceToHost, s));
+    CU(cudaStreamSynchronize(s));
+    // r as jb_metric_feature_pearson finishes it (x = the prediction, y = the target); a constant column gives nan
+    auto pearson = [&](const double* q, long long c) {
+      const double st = tacc[2 * c], stt = tacc[2 * c + 1];
+      const double cxy = q[2] - q[0] * st / N, cxx = q[1] - q[0] * q[0] / N, cyy = stt - st * st / N;
+      return cxy / std::sqrt(cxx * cyy);
+    };
+    if (j0 == 0 && target)
+      for (long long c = 0; c < d_out; ++c) base_r[c] = pearson(&acc[static_cast<size_t>(c) * 4], c);
+    for (long long q = 0; q < na; ++q)
+      for (long long c = 0; c < d_out; ++c) {
+        const double* v = &acc[(static_cast<size_t>(q + 1) * d_out + c) * 4];
+        shift[(j0 + q) * d_out + c] = v[3] / N;
+        if (target) r[(j0 + q) * d_out + c] = pearson(v, c);
+      }
+  }
   return 0;
 }
 

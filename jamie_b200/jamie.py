@@ -682,6 +682,14 @@ class JAMIE(UnionCom):
             return eng.encode(i, np.asarray(rows, np.float32), self._stream())
         return shard_rows_apply(run, data)
 
+    def feature_impact(self, data, modality, target=None, features=None, fill='mean', space='output'):
+        """Rank the raw input features of ``data`` (modality ``modality``) by ablation: each feature in turn set to ``fill``
+        ('mean' of its column, a scalar or one value per feature), scored against ``target`` (the measured other modality)
+        or by how far the predictions (``space='output'``) or embeddings (``space='latent'``) move. Runs on the GPU without
+        a host round trip per feature; returns an ``impact.FeatureImpact``."""
+        from .impact import feature_impact
+        return feature_impact(self, data, modality, target=target, features=features, fill=fill, space=space)
+
     # ------------------------------------------------------------------------------------------------ metrics
     def test_closer(self, integrated_data, distance_metric=None):
         """Test fraction of samples closer than the true match (jamie/jamie.py:892-913; prints ``foscttm: ...``)"""
