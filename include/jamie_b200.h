@@ -208,6 +208,30 @@ int jb_feature_impact(jb_engine* e, int from, int to, const double* Z, long long
                       const double* aff_scale, const double* aff_shift, long long d_out, const float* target, double* base_r,
                       double* r, double* shift, long long batch_bytes, void* stream);
 
+/* Shapley values by antithetic permutation walks (SURVEY.md 3.2: the notebooks' SHAP explainers around modal_predict;
+ * jamie_b200/shapley.py). For every explained row x, permutation pi and background row b, the walk from b to x adds the
+ * raw features in the order pi; with a linear input map its network inputs are z_t = z_{t-1} + (x_j - b_j) w_j, j = pi_t,
+ * z_0 = z_b, built on the device in float64 and rounded once to fp32 per row. A step with x_j == b_j gets no chain row.
+ *   X [nx, d], B [nb, d] float64 host: raw explained and background rows.  Zb [nb, dims[from]] float64: preprocessing[from](B).
+ *   perms [n_perm, d] int32: permutations of the d raw features.
+ *   w     w_col == NULL: [d, dims[from]] (components_[:, j] / s of a PCA input side);
+ *         else [d] scalars added to column w_col[j] only (1 / s_j of a side standardised per column).
+ * y = map(chain(z)), chain and output map as jb_feature_impact, restricted to n_out selected outputs: map_kind 1 takes comp
+ * [D_to, n_out] and mean [n_out] already restricted to them; kinds 0 / 2 take out_cols [n_out] (columns of the chain's
+ * output; kind 2's aff_scale / aff_shift have the chain's width).
+ *   phi [nx, d, n_out] += sum over (permutation, background row) of y(z_t) - y(z_{t-1}), credited to feature pi_t.
+ *   base [n_out] += sum over b of y(z_b).  stats [2] (or NULL) += {chain rows of the walks, inactive steps skipped}.
+ * The caller divides by n_perm * nb. Works in batches of (explained row, background row) segments whose working set stays
+ * under batch_bytes (and the free memory); no chain row leaves the device. Each accumulator of phi receives its terms one
+ * at a time in float64, in (permutation, background row) order, without atomics: results are bit-identical across reruns
+ * and for any batch_bytes. Refuses, before any allocation, a problem whose smallest batch (one segment of d active steps)
+ * does not fit in free device memory. Host pointers; synchronous. */
+int jb_shapley(jb_engine* e, int from, int to, const double* X, long long nx, const double* B, long long nb, long long d,
+               const double* Zb, const int* perms, long long n_perm, const double* w, const int* w_col, int map_kind,
+               const float* comp, const float* mean, float m, float s, const double* aff_scale, const double* aff_shift,
+               const int* out_cols, long long n_out, double* phi, double* base, long long* stats, long long batch_bytes,
+               void* stream);
+
 /* PCA fit (jamie/jamie.py:436-452, sklearn PCA(n_components).fit with the covariance_eigh solver): the two O(n d) /
  * O(n d^2) passes over the [n, d] matrix run on the GPU -- column sums, then the centred Gram matrix
  * (X - mean)^T (X - mean) as a split (fp32-class) tensor-core GEMM accumulated over row chunks in float64. The caller

@@ -95,6 +95,8 @@ SIGNATURES = {
     'jb_pca_inverse': (C.c_int, [_P, _P, _LL, C.c_int, _P, _P, _LL, C.c_float, C.c_float, _P, C.c_int, _P]),
     'jb_feature_impact': (C.c_int, [_P, C.c_int, C.c_int, _P, _LL, _LL, _P, _P, _P, C.c_int, _P, _P, C.c_float, C.c_float,
                                     _P, _P, _LL, _P, _P, _P, _P, _LL, _P]),
+    'jb_shapley': (C.c_int, [_P, C.c_int, C.c_int, _P, _LL, _P, _LL, _LL, _P, _P, _LL, _P, _P, C.c_int, _P, _P, C.c_float,
+                             C.c_float, _P, _P, _P, _LL, _P, _P, _P, _LL, _P]),
     'jb_debug_read': (_LL, [_P, C.c_char_p, _P, _LL]),
     'jb_launch_count': (_LL, [_P]),
 }

@@ -36,6 +36,7 @@
 #include "distances.cuh"
 #include "pcaop.cuh"
 #include "impact.cuh"
+#include "shapley.cuh"
 
 namespace {
 
@@ -1789,6 +1790,154 @@ int jb_feature_impact(jb_engine* e, int from, int to, const double* Z, long long
         shift[(j0 + q) * d_out + c] = v[3] / N;
         if (target) r[(j0 + q) * d_out + c] = pearson(v, c);
       }
+  }
+  return 0;
+}
+
+// ---------------------------------------------------------------------------------------------- Shapley values (SURVEY 3.2)
+
+int jb_shapley(jb_engine* e, int from, int to, const double* X, long long nx, const double* B, long long nb, long long d,
+               const double* Zb, const int* perms, long long n_perm, const double* w, const int* w_col, int map_kind,
+               const float* comp, const float* mean, float m, float sdev, const double* aff_scale, const double* aff_shift,
+               const int* out_cols, long long n_out, double* phi, double* base, long long* stats, long long batch_bytes,
+               void* stream) {
+  if (!e || !X || !B || !Zb || !perms || !w || !phi || !base) return fail("null argument");
+  if (from < 0 || from > 1 || to < -1 || to > 1) return fail("modality index out of range");
+  if (nx <= 0 || nb <= 0 || d <= 0 || n_perm <= 0 || n_out <= 0) return fail("bad Shapley shape");
+  if (d > 8LL * 65535 || n_out > 32LL * 65535 || nx * nb > (1LL << 31) - 1) return fail("Shapley problem too large to index");
+  const int D_in = e->D[from];
+  const int D_to = to < 0 ? e->L : e->D[to];
+  if (map_kind == 1) {
+    if (!comp || !mean || to < 0) return fail("the PCA output map needs comp, mean and an output modality");
+  } else if (map_kind == 0 || map_kind == 2) {
+    if (!out_cols) return fail("output map %d needs the selected output columns", map_kind);
+    if (map_kind == 2 && (!aff_scale || !aff_shift)) return fail("the per-column output map needs %d scales and shifts", D_to);
+    if (n_out > D_to) return fail("%lld output columns selected, the network gives %d", n_out, D_to);
+    for (long long o = 0; o < n_out; ++o)
+      if (out_cols[o] < 0 || out_cols[o] >= D_to) return fail("output column %d out of range [0, %d)", out_cols[o], D_to);
+  } else {
+    return fail("unknown output map %d", map_kind);
+  }
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const long long S_all = nx * nb;
+  const int di = static_cast<int>(d);
+  const long long Q = (d + jb::SHP_TC - 1) / jb::SHP_TC;
+  const long long ldin = r4(D_in), ldto = r4(D_to), ldo = r4(static_cast<int>(n_out)), ldk = r4(D_to);
+  // bytes per chain row (walk row, chain output, and for PCA the split planes and the inverse's output), per segment of a
+  // batch (chunk sums, chunk counts and offsets, step -> row map), and fixed (raw rows, z_b, w, permutations, phi, f(b))
+  const double row_b = 4.0 * (ldin + ldto + (map_kind == 1 ? 2.0 * ldk + ldo : 0.0));
+  const double seg_b = 8.0 * Q * D_in + 8.0 * Q + 4.0 * d + 4.0;
+  const double fixed = 8.0 * (nx + nb) * d + 8.0 * nb * D_in + 4.0 * n_perm * d + (w_col ? 12.0 * d : 8.0 * d * D_in) +
+                       8.0 * nx * d * n_out + 4.0 * nb * n_out + 16.0 * S_all + 12.0 * n_out +
+                       (map_kind == 1 ? 12.0 * D_to * ldo + 4.0 * n_out : 0.0) + (map_kind == 2 ? 16.0 * D_to : 0.0);
+  size_t free_b = 0, total_b = 0;
+  CU(cudaMemGetInfo(&free_b, &total_b));
+  const double avail = static_cast<double>(free_b) - (256.0 * (1 << 20));   // GEMM tables, tensor maps, allocator slack
+  const double need_min = fixed + d * row_b + seg_b;                         // one segment, every step active
+  if (need_min > avail)
+    return fail("Shapley values need %.2f GB of device memory for their smallest batch (one segment of %lld steps); "
+                "%.2f GB free", need_min / 1e9, d, static_cast<double>(free_b) / 1e9);
+  const double budget = static_cast<double>(batch_bytes) < avail - fixed ? static_cast<double>(batch_bytes) : avail - fixed;
+  if (prepare_eval(e, s)) return 1;
+
+  DevArr<double> dX, dB, dZb, dW, dPhi, dBase, dSc, dSh, dPart;
+  DevArr<int> dPerm, dWc, dOc, dCcnt, dCoff, dFirst, dRowof;
+  DevArr<long long> dCnt;
+  DevArr<float> dFB;
+  DevBuf xin, cout, zhi, zlo, o;
+  PcaInverse inv;
+  if (dX.upload(X, static_cast<size_t>(nx) * d) || dB.upload(B, static_cast<size_t>(nb) * d) ||
+      dZb.upload(Zb, static_cast<size_t>(nb) * D_in) || dPerm.upload(perms, static_cast<size_t>(n_perm) * d) ||
+      (w_col ? (dW.upload(w, d) || dWc.upload(w_col, d)) : dW.upload(w, static_cast<size_t>(d) * D_in)) ||
+      dPhi.upload(phi, static_cast<size_t>(nx) * d * n_out) || dBase.upload(base, n_out) ||
+      dFB.alloc(static_cast<size_t>(nb) * n_out) || dCnt.alloc(S_all)) return 1;
+  if (map_kind != 1 && dOc.upload(out_cols, n_out)) return 1;
+  if (map_kind == 2 && (dSc.upload(aff_scale, D_to) || dSh.upload(aff_shift, D_to))) return 1;
+  if (map_kind == 1 && inv.prepare(e, comp, mean, D_to, n_out, m, sdev, s)) return 1;
+
+  // chain rows per segment (the same for every permutation), then batches: runs of segments in order whose rows and
+  // per-segment buffers fit the budget; a segment is never split
+  jb::k_shap_count<<<static_cast<unsigned>(S_all), 256, 0, s>>>(dX.p, dB.p, di, static_cast<int>(nb), dCnt.p); ++e->launches;
+  CU(cudaGetLastError());
+  std::vector<long long> cnt(S_all);
+  CU(cudaMemcpyAsync(cnt.data(), dCnt.p, S_all * sizeof(long long), cudaMemcpyDeviceToHost, s));
+  CU(cudaStreamSynchronize(s));
+  struct Batch { long long s0, S, rows; };
+  std::vector<Batch> batches;
+  long long Smax = 1, Rmax = 0, total_rows = 0;
+  for (long long g = 0; g < S_all;) {
+    Batch bt{g, 0, 0};
+    while (g < S_all && (bt.S == 0 || ((bt.rows + cnt[g]) * row_b + (bt.S + 1) * seg_b <= budget &&
+                                       bt.rows + cnt[g] <= (1LL << 30) && bt.S < (1LL << 24)))) {
+      bt.rows += cnt[g++];
+      ++bt.S;
+    }
+    batches.push_back(bt);
+    Smax = bt.S > Smax ? bt.S : Smax;
+    Rmax = bt.rows > Rmax ? bt.rows : Rmax;
+    total_rows += bt.rows;
+  }
+  const long long Rb = nb < d ? nb : d;   // rows per chunk of the f(b) pass
+  const long long R = Rmax > Rb ? Rmax : Rb;
+  if (xin.alloc(static_cast<size_t>(R) * ldin) || cout.alloc(static_cast<size_t>(R) * ldto) ||
+      dPart.alloc(static_cast<size_t>(Smax) * Q * D_in) || dCcnt.alloc(static_cast<size_t>(Smax) * Q) ||
+      dCoff.alloc(static_cast<size_t>(Smax) * Q) || dFirst.alloc(Smax) || dRowof.alloc(static_cast<size_t>(Smax) * d)) return 1;
+  if (map_kind == 1 && (zhi.alloc(static_cast<size_t>(R) * inv.ldk) || zlo.alloc(static_cast<size_t>(R) * inv.ldk) ||
+                        o.alloc(static_cast<size_t>(R) * ldo))) return 1;
+  // the chain (and for PCA the inverse) of `rows` walk rows in xin; the mapped outputs are then read through ShapOut
+  auto chain = [&](long long rows, jb::ShapOut* out) -> int {
+    if (eval_common(e, from, to, xin.p, rows, ldin, cout.p, ldto, 1, s)) return 1;
+    *out = jb::ShapOut{cout.p, ldto, map_kind, dOc.p, dSc.p, dSh.p};
+    if (map_kind == 1) {
+      if (inv.apply(e, cout.p, ldto, rows, zhi.p, zlo.p, o.p, s)) return 1;
+      out->Y = o.p;
+      out->ldy = ldo;
+    }
+    return 0;
+  };
+  const unsigned ogrid = static_cast<unsigned>((n_out + 127) / 128);
+  for (long long b0 = 0; b0 < nb; b0 += Rb) {   // f(b) and base += sum_b f(b)
+    const long long rows = nb - b0 < Rb ? nb - b0 : Rb;
+    jb::k_shap_rows_f32<<<static_cast<unsigned>(rows), 128, 0, s>>>(dZb.p, D_in, b0, xin.p, ldin); ++e->launches;
+    jb::ShapOut Y{};
+    if (chain(rows, &Y)) return 1;
+    jb::k_shap_base<<<ogrid, 128, 0, s>>>(Y, static_cast<int>(rows), b0, static_cast<int>(n_out), dFB.p, dBase.p); ++e->launches;
+  }
+  std::vector<int> first(Smax);
+  for (long long p = 0; p < n_perm; ++p) {
+    const int* perm = dPerm.p + p * d;
+    for (const Batch& bt : batches) {
+      if (bt.rows == 0) continue;
+      const int S = static_cast<int>(bt.S);
+      long long r = 0;
+      for (long long i = 0; i < bt.S; ++i) { first[i] = static_cast<int>(r); r += cnt[bt.s0 + i]; }
+      CU(cudaMemcpyAsync(dFirst.p, first.data(), bt.S * sizeof(int), cudaMemcpyHostToDevice, s));
+      const dim3 wgrid(static_cast<unsigned>((S + jb::SHP_SG - 1) / jb::SHP_SG), static_cast<unsigned>(Q),
+                       static_cast<unsigned>((D_in + jb::SHP_CT - 1) / jb::SHP_CT));
+      jb::k_shap_walk<false><<<wgrid, jb::SHP_CT, 0, s>>>(dX.p, dB.p, di, static_cast<int>(nb), bt.s0, S, perm, dW.p, dWc.p,
+                                                          D_in, dPart.p, dCcnt.p, nullptr, nullptr, 0, nullptr); ++e->launches;
+      jb::k_shap_chunk_start<<<static_cast<unsigned>(S), 128, 0, s>>>(dZb.p, D_in, static_cast<int>(nb), bt.s0,
+                                                                      static_cast<int>(Q), dPart.p, dCcnt.p, dFirst.p,
+                                                                      dCoff.p); ++e->launches;
+      jb::k_shap_walk<true><<<wgrid, jb::SHP_CT, 0, s>>>(dX.p, dB.p, di, static_cast<int>(nb), bt.s0, S, perm, dW.p, dWc.p,
+                                                         D_in, dPart.p, nullptr, dCoff.p, xin.p, ldin, dRowof.p); ++e->launches;
+      jb::ShapOut Y{};
+      if (chain(bt.rows, &Y)) return 1;
+      const long long xa = bt.s0 / nb, xb = (bt.s0 + bt.S - 1) / nb;
+      const dim3 fgrid(static_cast<unsigned>(xb - xa + 1), static_cast<unsigned>((d + 7) / 8),
+                       static_cast<unsigned>((n_out + 31) / 32));
+      jb::k_shap_fold<<<fgrid, dim3(32, 8), 0, s>>>(Y, dFB.p, dRowof.p, dFirst.p, perm, di, static_cast<int>(nb), bt.s0, S,
+                                                    static_cast<int>(n_out), dPhi.p); ++e->launches;
+      // `first` is reused by the next batch: its pageable copy has been staged by the driver on return, as in eval_common
+    }
+  }
+  CU(cudaGetLastError());
+  CU(cudaMemcpyAsync(phi, dPhi.p, static_cast<size_t>(nx) * d * n_out * sizeof(double), cudaMemcpyDeviceToHost, s));
+  CU(cudaMemcpyAsync(base, dBase.p, static_cast<size_t>(n_out) * sizeof(double), cudaMemcpyDeviceToHost, s));
+  CU(cudaStreamSynchronize(s));
+  if (stats) {
+    stats[0] += n_perm * total_rows;
+    stats[1] += n_perm * (S_all * d - total_rows);
   }
   return 0;
 }

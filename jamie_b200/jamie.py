@@ -690,6 +690,16 @@ class JAMIE(UnionCom):
         from .impact import feature_impact
         return feature_impact(self, data, modality, target=target, features=features, fill=fill, space=space)
 
+    def shap_values(self, data, modality, background, outputs=None, space='output', n_permutations=2, seed=None):
+        """Shapley values of the raw input features of ``data`` (modality ``modality``) for the imputed columns ``outputs``
+        of the other modality (``space='output'``, default all) or the embedding dims (``space='latent'``), against the
+        raw rows ``background``: antithetic permutation sampling with ``n_permutations`` permutations drawn from ``seed``
+        (default ``manual_seed``). Runs on the GPU without a host round trip per masked batch; returns a
+        ``shapley.ShapValues`` (values [n, d_in, |outputs|], base_values, outputs)."""
+        from .shapley import shap_values
+        return shap_values(self, data, modality, background, outputs=outputs, space=space, n_permutations=n_permutations,
+                           seed=seed)
+
     # ------------------------------------------------------------------------------------------------ metrics
     def test_closer(self, integrated_data, distance_metric=None):
         """Test fraction of samples closer than the true match (jamie/jamie.py:892-913; prints ``foscttm: ...``)"""
