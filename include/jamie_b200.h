@@ -250,12 +250,25 @@ int jb_pca_gram(jb_engine* e, const float* X, long long n, long long d, const do
  *     every query row the majority class (uniform votes; ties to the lowest class index) of its k nearest reference rows
  *     (euclidean; equal distances by the lowest row index). ref_class: class indices in [0, n_classes).
  *   jb_metric_feature_pearson: per-feature Pearson r of two [n, d] matrices (jamie/evaluation.py:491-513, sklearn
- *     r_regression); a constant feature gives nan. */
+ *     r_regression); a constant feature gives nan.
+ *   jb_metric_feature_auroc: per-feature AUROC of imputed scores against present / absent measured values (the AUROC
+ *     panel of jamie/evaluation.py:468-490, sklearn roc_auc_score(measured[:, j] > threshold, imputed[:, j])). scores:
+ *     [n, d] row-major fp32 (finite; -0.0 and +0.0 are one score). The positives of column j are the rows
+ *     pos_row[pos_ptr[j] .. pos_ptr[j + 1]) (CSC lists: int64 pos_ptr [d + 1] from 0, int32 rows increasing in [0, n));
+ *     every other row is a negative. Rows are grouped by equal score in ascending order; for group g with pos_g
+ *     positives, neg_g negatives and negbefore_g negatives in all lower groups,
+ *       u2[j] = 2U = sum_g pos_g (2 negbefore_g + neg_g)   (exact, uint64; n < 2^31),   n_pos[j] = P,
+ *     and AUROC = 2U / (2 P N) with N = n - P (one float64 division by the caller; P = 0 or N = 0 has no AUROC).
+ *     Integer arithmetic only: results do not depend on batch_bytes. Works in column batches whose working set stays
+ *     under batch_bytes (and the free memory); refuses, before any allocation, a problem whose one-column batch does not
+ *     fit in free device memory. */
 int jb_metric_foscttm(const float* emb0, const float* emb1, long long n, int L, int device,
                       unsigned long long* raw_count_closer);
 int jb_metric_knn_vote(const float* query, long long nq, const float* ref, const int* ref_class, long long nr, int L,
                        int k, int n_classes, int device, int* pred_class);
 int jb_metric_feature_pearson(const float* x, const float* y, long long n, long long d, int device, double* r);
+int jb_metric_feature_auroc(const float* scores, long long n, long long d, const long long* pos_ptr, const int* pos_row,
+                            long long batch_bytes, int device, unsigned long long* u2, long long* n_pos);
 
 /* Distances of the F estimation (compute_distances, jamie/jamie.py:839-890; the default distance_mode 'geodesic' is
  * unioncom.utils.geodesic_distances of unioncom==0.4.0, restated and unpinned in jamie_b200/correspondence.py).

@@ -37,6 +37,7 @@
 #include "pcaop.cuh"
 #include "impact.cuh"
 #include "shapley.cuh"
+#include "auroc.cuh"
 
 namespace {
 
@@ -2005,6 +2006,106 @@ int jb_metric_feature_pearson(const float* x, const float* y, long long n, long 
     const double cxy = m[4] - m[0] * m[1] / N, cxx = m[2] - m[0] * m[0] / N, cyy = m[3] - m[1] * m[1] / N;
     r[c] = cxy / std::sqrt(cxx * cyy);   // constant feature: 0 / 0 = nan, as the host definition gives
   }
+  return 0;
+}
+
+namespace {
+struct AurocStreams {   // compute and copy streams of jb_metric_feature_auroc; synchronised before the buffers are freed
+  cudaStream_t s = nullptr, sc = nullptr;
+  cudaEvent_t copied = nullptr, keyed = nullptr, done[2] = {nullptr, nullptr};
+  int create() {
+    CU(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
+    CU(cudaStreamCreateWithFlags(&sc, cudaStreamNonBlocking));
+    for (cudaEvent_t* ev : {&copied, &keyed, &done[0], &done[1]}) CU(cudaEventCreateWithFlags(ev, cudaEventDisableTiming));
+    return 0;
+  }
+  ~AurocStreams() {
+    if (s) cudaStreamSynchronize(s);
+    if (sc) cudaStreamSynchronize(sc);
+    for (cudaEvent_t ev : {copied, keyed, done[0], done[1]})
+      if (ev) cudaEventDestroy(ev);
+    if (s) cudaStreamDestroy(s);
+    if (sc) cudaStreamDestroy(sc);
+  }
+};
+}  // namespace
+
+int jb_metric_feature_auroc(const float* scores, long long n, long long d, const long long* pos_ptr, const int* pos_row,
+                            long long batch_bytes, int device, unsigned long long* u2, long long* n_pos) {
+  if (!scores || !pos_ptr || !u2 || !n_pos) return fail("null argument");
+  if (n <= 0 || d <= 0 || n > (1LL << 31) - 1) return fail("bad matrix shape: %lld rows, %lld columns", n, d);
+  CU(cudaSetDevice(device));
+  const bool shared = n <= jb::AU_SMEM_ROWS;
+  // bytes per column of a batch: the fp32 slab, its keys, two buffers of positive lists (n rows each at most) and, above
+  // the shared-memory regime, the sort's two key buffers
+  const double col_b = (shared ? 16.0 : 24.0) * static_cast<double>(n);
+  const double fixed = 16.0 * static_cast<double>(d) + 8.0;
+  size_t free_b = 0, total_b = 0;
+  CU(cudaMemGetInfo(&free_b, &total_b));
+  const double avail = static_cast<double>(free_b) - (64.0 * (1 << 20));
+  if (fixed + col_b > avail)
+    return fail("AUROC needs %.2f GB of device memory for one column of %lld rows; %.2f GB free", (fixed + col_b) / 1e9, n,
+                static_cast<double>(free_b) / 1e9);
+  if (pos_ptr[0] != 0 || (pos_ptr[d] > 0 && !pos_row)) return fail("bad positive lists");
+  for (long long c = 0; c < d; ++c) {
+    const long long a = pos_ptr[c], b = pos_ptr[c + 1];
+    if (b < a || b - a > n) return fail("column %lld has %lld positives in %lld rows", c, b - a, n);
+    for (long long i = a; i < b; ++i)
+      if (pos_row[i] < 0 || pos_row[i] >= n || (i > a && pos_row[i] <= pos_row[i - 1]))
+        return fail("the positive rows of column %lld must increase and lie in [0, %lld)", c, n);
+    n_pos[c] = b - a;
+  }
+  const double budget = static_cast<double>(batch_bytes) < avail - fixed ? static_cast<double>(batch_bytes) : avail - fixed;
+  long long w = static_cast<long long>(budget / col_b);
+  if (w < 1) w = 1;
+  if (w > d) w = d;
+  if (w > 65535LL * 32) w = 65535LL * 32;   // column tiles of k_auroc_keys in grid.y
+  long long lmax = 0;                        // the largest batch's positive lists
+  for (long long j0 = 0; j0 < d; j0 += w) {
+    const long long j1 = j0 + w < d ? j0 + w : d;
+    lmax = pos_ptr[j1] - pos_ptr[j0] > lmax ? pos_ptr[j1] - pos_ptr[j0] : lmax;
+  }
+  if (shared) CU(cudaFuncSetAttribute(jb::k_auroc_col<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 8 * jb::AU_SMEM_ROWS));
+
+  DevArr<long long> dPtr;
+  DevArr<unsigned long long> dU2;
+  DevArr<float> slab;
+  DevArr<uint32_t> keys, scratch;
+  DevArr<int> rows[2];
+  if (dPtr.upload(pos_ptr, static_cast<size_t>(d) + 1) || dU2.alloc(d) || slab.alloc(static_cast<size_t>(n) * w) ||
+      keys.alloc(static_cast<size_t>(n) * w) || rows[0].alloc(lmax) || rows[1].alloc(lmax) ||
+      (!shared && scratch.alloc(static_cast<size_t>(2 * n) * w))) return 1;
+  AurocStreams st;   // declared after the buffers: its destructor synchronises before they are freed
+  if (st.create()) return 1;
+  // batch b: the copy stream uploads the slab once batch b - 1 has been keyed and the lists once batch b - 2 is done, so
+  // that the host-to-device copy of one batch overlaps the sort of the previous one
+  int b = 0;
+  for (long long j0 = 0; j0 < d; j0 += w, ++b) {
+    const long long wb = d - j0 < w ? d - j0 : w;
+    const long long l0 = pos_ptr[j0], nl = pos_ptr[j0 + wb] - l0;
+    long long pcap = 0;
+    for (long long c = j0; c < j0 + wb; ++c) pcap = n_pos[c] > pcap ? n_pos[c] : pcap;
+    CU(cudaStreamWaitEvent(st.sc, st.keyed, 0));
+    CU(cudaMemcpy2DAsync(slab.p, static_cast<size_t>(wb) * 4, scores + j0, static_cast<size_t>(d) * 4, static_cast<size_t>(wb) * 4,
+                         static_cast<size_t>(n), cudaMemcpyHostToDevice, st.sc));
+    CU(cudaStreamWaitEvent(st.sc, st.done[b & 1], 0));
+    if (nl > 0) CU(cudaMemcpyAsync(rows[b & 1].p, pos_row + l0, static_cast<size_t>(nl) * 4, cudaMemcpyHostToDevice, st.sc));
+    CU(cudaEventRecord(st.copied, st.sc));
+    CU(cudaStreamWaitEvent(st.s, st.copied, 0));
+    jb::k_auroc_keys<<<dim3(static_cast<unsigned>((n + 31) / 32), static_cast<unsigned>((wb + 31) / 32)), dim3(32, 8), 0, st.s>>>(
+        slab.p, n, static_cast<int>(wb), keys.p);
+    CU(cudaEventRecord(st.keyed, st.s));
+    if (shared)
+      jb::k_auroc_col<true><<<static_cast<unsigned>(wb), jb::AU_THREADS, static_cast<size_t>(pcap) * 8, st.s>>>(
+          keys.p, n, dPtr.p + j0, rows[b & 1].p, static_cast<int>(pcap), nullptr, dU2.p + j0);
+    else
+      jb::k_auroc_col<false><<<static_cast<unsigned>(wb), jb::AU_THREADS, 0, st.s>>>(keys.p, n, dPtr.p + j0, rows[b & 1].p, 0,
+                                                                                   scratch.p, dU2.p + j0);
+    CU(cudaEventRecord(st.done[b & 1], st.s));
+  }
+  CU(cudaGetLastError());
+  CU(cudaMemcpyAsync(u2, dU2.p, static_cast<size_t>(d) * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st.s));
+  CU(cudaStreamSynchronize(st.s));
   return 0;
 }
 

@@ -1,11 +1,13 @@
 """The acceptance metrics the reference's notebooks report, with the reference's own definitions (same denominators,
 same default k, same printed lines), computed on the GPU (SURVEY.md 8 row N4): the O(n^2 L) distance work of FOSCTTM and
-of the kNN label transfer, and the per-feature correlation of an imputed matrix, run as CUDA kernels behind the C ABI
-(``jb_metric_foscttm``, ``jb_metric_knn_vote``, ``jb_metric_feature_pearson``: csrc/metrics.cuh).
+of the kNN label transfer, and the per-feature correlation and AUROC of an imputed matrix, run as CUDA kernels behind the
+C ABI (``jb_metric_foscttm``, ``jb_metric_knn_vote``, ``jb_metric_feature_pearson``: csrc/metrics.cuh;
+``jb_metric_feature_auroc``: csrc/auroc.cuh).
 
 Reference: FOSCTTM ``test_closer`` jamie/evaluation.py:65-85 (class method jamie/jamie.py:892-913), label-transfer
 accuracy ``test_LabelTA`` jamie/evaluation.py:114-132 (class method jamie/jamie.py:943-961: k = None default), per-feature
-imputation correlation jamie/evaluation.py:491-513 (sklearn ``r_regression``).
+imputation correlation jamie/evaluation.py:491-513 (sklearn ``r_regression``) and AUROC jamie/evaluation.py:468-490
+(sklearn ``roc_auc_score`` on measured > threshold).
 
 There is no host fallback: without the CUDA library these functions raise.  The only host-side distance computation left
 is the reference's ``distance_metric=`` hook of ``test_closer`` (a user callable on the concatenated embeddings).
@@ -109,3 +111,86 @@ def mean_feature_r(imputed, measured):
     y = np.asarray(measured)
     keep = np.array([len(np.unique(col)) > 1 for col in y.T])
     return float(np.nanmean(imputation_correlation(imputed, measured)[keep]))
+
+
+# Upper bound of the device working set of one column batch of imputation_auroc (and of the host's temporaries while it
+# builds the positive lists of a dense ``measured``), in bytes.
+BATCH_BYTES = 1 << 30
+
+
+def _is_sparse(x):
+    return hasattr(x, 'tocsc') and not isinstance(x, np.ndarray)
+
+
+def positive_lists(measured, threshold, batch_bytes):
+    """The rows with measured > threshold of every column as CSC lists: (int64 ptr [d + 1], int32 rows, increasing within
+    a column). A scipy.sparse ``measured`` is read through its CSC form and never densified (threshold >= 0: implicit
+    zeros are negatives); a dense one in column blocks of about batch_bytes / 4 elements. Raises ValueError for
+    non-finite values."""
+    n, d = measured.shape
+    if _is_sparse(measured):
+        M = measured.tocsc(copy=True)
+        M.sum_duplicates()                      # the values a dense copy would hold, rows increasing within a column
+        if not np.isfinite(M.data).all():
+            raise ValueError('measured has non-finite values')
+        keep = M.data > threshold
+        ck = np.concatenate([[0], np.cumsum(keep, dtype=np.int64)])
+        return ck[M.indptr], np.ascontiguousarray(M.indices[keep], np.int32)
+    counts, rows = np.zeros(d + 1, np.int64), []
+    cb = max(1, min(d, batch_bytes // (4 * max(n, 1))))
+    for j0 in range(0, d, cb):
+        blk = measured[:, j0:j0 + cb]
+        if not np.isfinite(blk).all():
+            raise ValueError('measured has non-finite values')
+        m = np.ascontiguousarray((blk > threshold).T)    # [columns, n]: nonzeros by column, then row
+        counts[j0 + 1:j0 + 1 + m.shape[0]] = m.sum(axis=1)
+        rows.append((np.flatnonzero(m) % n).astype(np.int32))
+    return np.cumsum(counts), np.concatenate(rows) if rows else np.zeros(0, np.int32)
+
+
+def imputation_auroc(imputed, measured, threshold=0.0, device=None):
+    """Per-feature AUROC of imputed values against the measured ones read as present / absent:
+    roc_auc_score(measured[:, j] > threshold, float32(imputed[:, j])) for every column j (the AUROC panel of
+    jamie/evaluation.py:468-490), computed on the GPU (``jb_metric_feature_auroc``) as the exact Mann-Whitney statistic
+    2U in integers, then one float64 division 2U / (2 P N). A column with one class only gives nan.
+
+    ``imputed`` is a dense [n, d] array (rounded to float32, as ``imputation_correlation`` does); ``measured`` is dense or
+    any scipy.sparse format (never densified). Labels compare ``measured`` as given with ``threshold``."""
+    if _is_sparse(imputed):
+        raise ValueError('imputed must be a dense array')
+    x = np.asarray(imputed)
+    y = measured if _is_sparse(measured) else np.asarray(measured)
+    if x.ndim != 2 or y.ndim != 2 or x.shape != y.shape:
+        raise ValueError(f'imputed and measured must be two [n, d] matrices of one shape, got {x.shape} and {y.shape}')
+    n, d = x.shape
+    if n >= 1 << 31:
+        raise ValueError(f'{n} rows: imputation_auroc takes fewer than 2^31')
+    if np.ndim(threshold) != 0:
+        raise ValueError('threshold must be a scalar')
+    try:
+        finite = np.isfinite(threshold)
+    except TypeError:
+        finite = False
+    if not finite:
+        raise ValueError(f'threshold must be a finite number, not {threshold!r}')
+    if _is_sparse(y) and threshold < 0:
+        raise ValueError('a sparse measured matrix with threshold < 0 would make every implicit zero positive: '
+                         'pass a dense array')
+    if n == 0:
+        raise ValueError('imputation_auroc needs at least one row')
+    with np.errstate(over='ignore'):
+        scores = _f32(x)
+    if not np.isfinite(scores).all():
+        raise ValueError('imputed has non-finite values (after rounding to float32)')
+    ptr, rows = positive_lists(y, threshold, BATCH_BYTES)
+    if d == 0:
+        return np.zeros(0, np.float64)
+    u2 = np.empty(d, np.uint64)
+    n_pos = np.empty(d, np.int64)
+    lib = _lib.load()
+    p = lambda a: a.ctypes.data_as(C.c_void_p)   # noqa: E731
+    _lib.check(lib.jb_metric_feature_auroc(p(scores), n, d, p(ptr), p(rows), int(BATCH_BYTES), _device(device), p(u2),
+                                           p(n_pos)))
+    # 2U and 2PN are exact integers; Python's int division rounds their quotient correctly
+    return np.array([u / (2 * q * (n - q)) if 0 < q < n else np.nan for u, q in zip(u2.tolist(), n_pos.tolist())],
+                    np.float64)
