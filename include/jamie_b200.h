@@ -270,6 +270,26 @@ int jb_metric_feature_pearson(const float* x, const float* y, long long n, long 
 int jb_metric_feature_auroc(const float* scores, long long n, long long d, const long long* pos_ptr, const int* pos_row,
                             long long batch_bytes, int device, unsigned long long* u2, long long* n_pos);
 
+/* Exact kNN search and kNN averaging on the GPU (csrc/knn.cuh; no engine handle; host pointers in, synchronous). They
+ * replace sklearn's NearestNeighbors(algorithm='brute').kneighbors and KNeighborsRegressor(algorithm='brute').predict on
+ * the host, whose search grows with nq * nr.
+ *   jb_knn: for every query row the k nearest reference rows in euclidean distance. query [nq, L], ref [nr, L] row-major
+ *     fp32; distances are float64 sums of squared fp32 differences (sequential over the columns, the tile arithmetic of
+ *     jb_metric_foscttm). idx [nq, k] int64 and dist [nq, k] float64 (sqrt of the sum; NULL = not wanted) in ascending
+ *     (squared sum, reference index) order: equal distances by the lowest index, as a stable argsort gives. 1 <= k <=
+ *     min(1024, nr); nq, nr < 2^31. No [nq, nr] matrix is formed: the reference rows stay on the device, the queries go in
+ *     batches whose lists fit in batch_bytes, and a small batch splits the reference rows into ranges whose lists are
+ *     merged. No floating-point atomics: results do not depend on batch_bytes or the device.
+ *   jb_knn_average: out[q, c] = sum_t w[q, t] values[idx[q, t], c] / sum_t w[q, t] in float64, summed in list order, for
+ *     idx [nq, k] int64 in [0, nr) (the lists of jb_knn), weights [nq, k] float64 or NULL (all 1), values [nr, w] float64
+ *     with row pitch ldv, out [nq, w] float64. The values go to the device in column slabs under batch_bytes.
+ *   Both refuse, before any allocation, a problem whose smallest batch (one query row; one column) does not fit in free
+ *   device memory. */
+int jb_knn(const float* query, long long nq, const float* ref, long long nr, int L, int k, long long batch_bytes, int device,
+           long long* idx, double* dist);
+int jb_knn_average(const long long* idx, const double* weights, long long nq, int k, const double* values, long long nr,
+                   long long w, long long ldv, long long batch_bytes, int device, double* out);
+
 /* Distances of the F estimation (compute_distances, jamie/jamie.py:839-890; the default distance_mode 'geodesic' is
  * unioncom.utils.geodesic_distances of unioncom==0.4.0, restated and unpinned in jamie_b200/correspondence.py).
  * A jb_dist handle owns one n x n float64 matrix D on one device and a stream; host pointers throughout.

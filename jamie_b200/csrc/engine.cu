@@ -38,6 +38,7 @@
 #include "impact.cuh"
 #include "shapley.cuh"
 #include "auroc.cuh"
+#include "knn.cuh"
 
 namespace {
 
@@ -2105,6 +2106,133 @@ int jb_metric_feature_auroc(const float* scores, long long n, long long d, const
   }
   CU(cudaGetLastError());
   CU(cudaMemcpyAsync(u2, dU2.p, static_cast<size_t>(d) * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st.s));
+  CU(cudaStreamSynchronize(st.s));
+  return 0;
+}
+
+// ---------------------------------------------------------------------------------------------- kNN search and average
+
+namespace {
+struct KnnStream {   // the stream of jb_knn / jb_knn_average; synchronised before the buffers are freed
+  cudaStream_t s = nullptr;
+  int create() { CU(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking)); return 0; }
+  ~KnnStream() {
+    if (s) { cudaStreamSynchronize(s); cudaStreamDestroy(s); }
+  }
+};
+double knn_avail() {   // free device memory less a margin for the context's own allocations
+  size_t free_b = 0, total_b = 0;
+  if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess) return 0.0;
+  return static_cast<double>(free_b) - (64.0 * (1 << 20));
+}
+}  // namespace
+
+int jb_knn(const float* query, long long nq, const float* ref, long long nr, int L, int k, long long batch_bytes, int device,
+           long long* idx, double* dist) {
+  if (!query || !ref || !idx) return fail("null argument");
+  if (nq <= 0 || nr <= 0 || L <= 0) return fail("bad embedding shape: %lld query rows, %lld reference rows, %d columns", nq, nr, L);
+  if (nq > INT_MAX || nr > INT_MAX) return fail("%lld query rows, %lld reference rows: jb_knn takes fewer than 2^31 of each", nq, nr);
+  if (k < 1 || k > jb::KN_MAXK || k > nr) return fail("k = %d neighbours: 1 <= k <= %d and k <= %lld reference rows", k, jb::KN_MAXK, nr);
+  CU(cudaSetDevice(device));
+  // device bytes: the reference rows (resident), and for each query row of a batch its fp32 row and output lists, and
+  // per reference range its two list arrays and their length
+  const double ref_b = 4.0 * static_cast<double>(nr) * L;
+  const double row_b = 4.0 * L + 16.0 * k, range_b = 24.0 * k + 8.0;
+  const double avail = knn_avail();
+  if (ref_b + row_b + range_b > avail)
+    return fail("kNN search needs %.2f GB of device memory for %lld reference rows and one query row; %.2f GB free",
+                (ref_b + row_b + range_b) / 1e9, nr, (avail > 0 ? avail : 0) / 1e9);
+  const double budget = static_cast<double>(batch_bytes) < avail - ref_b ? static_cast<double>(batch_bytes) : avail - ref_b;
+  long long nqb = static_cast<long long>(budget / (row_b + range_b));
+  if (nqb > nq) nqb = nq;
+  if (nqb >= jb::MT_TILE) nqb -= nqb % jb::MT_TILE;
+  if (nqb < 1) nqb = 1;
+  int sms = 148;
+  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
+  const long long target = 4LL * sms;   // blocks per batch: split the reference rows into ranges until a small batch has them
+  const long long tiles_r = (nr + jb::MT_TILE - 1) / jb::MT_TILE;
+  const long long min_tiles = 2 * ((k + jb::MT_TILE - 1) / jb::MT_TILE);   // per range: k rows and as many again to select from
+  auto ranges_for = [&](long long rows, long long cap_lists) {
+    const long long tq = (rows + jb::MT_TILE - 1) / jb::MT_TILE;
+    long long S = (target + tq - 1) / tq;
+    if (S > tiles_r / min_tiles) S = tiles_r / min_tiles;
+    if (S > cap_lists / rows) S = cap_lists / rows;
+    if (S < 1) S = 1;
+    return S;
+  };
+  long long fit = static_cast<long long>((budget - static_cast<double>(nqb) * row_b) / (static_cast<double>(nqb) * range_b));
+  const long long cap_lists = ranges_for(nqb, (fit > 1 ? fit : 1) * nqb) * nqb;   // (range, query) lists allocated
+  CU(cudaFuncSetAttribute(jb::k_knn_search, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(jb::KN_SMEM)));
+
+  DevArr<float> dr, dq;
+  DevArr<double> ld, odist;
+  DevArr<int> lj;
+  DevArr<int2> meta;
+  DevArr<long long> oidx;
+  if (dr.alloc(static_cast<size_t>(nr) * L) || dq.alloc(static_cast<size_t>(nqb) * L) || ld.alloc(static_cast<size_t>(cap_lists) * 2 * k) ||
+      lj.alloc(static_cast<size_t>(cap_lists) * 2 * k) || meta.alloc(cap_lists) || oidx.alloc(static_cast<size_t>(nqb) * k) ||
+      (dist && odist.alloc(static_cast<size_t>(nqb) * k))) return 1;
+  KnnStream st;   // declared after the buffers: its destructor synchronises before they are freed
+  if (st.create()) return 1;
+  CU(cudaMemcpyAsync(dr.p, ref, static_cast<size_t>(nr) * L * 4, cudaMemcpyHostToDevice, st.s));
+  for (long long q0 = 0; q0 < nq; q0 += nqb) {
+    const long long nb = nq - q0 < nqb ? nq - q0 : nqb;
+    long long S = ranges_for(nb, cap_lists);
+    const long long per = (tiles_r + S - 1) / S;
+    S = (tiles_r + per - 1) / per;   // no empty range
+    CU(cudaMemcpyAsync(dq.p, query + q0 * L, static_cast<size_t>(nb) * L * 4, cudaMemcpyHostToDevice, st.s));
+    jb::k_knn_search<<<dim3(static_cast<unsigned>((nb + jb::MT_TILE - 1) / jb::MT_TILE), static_cast<unsigned>(S)), jb::MT_THREADS,
+                       jb::KN_SMEM, st.s>>>(dq.p, nb, dr.p, nr, L, k, per, ld.p, lj.p, meta.p);
+    jb::k_knn_merge<<<static_cast<unsigned>(nb), jb::KM_THREADS, 0, st.s>>>(ld.p, lj.p, meta.p, static_cast<int>(S), nb, k, oidx.p,
+                                                                           dist ? odist.p : nullptr);
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(idx + q0 * k, oidx.p, static_cast<size_t>(nb) * k * 8, cudaMemcpyDeviceToHost, st.s));
+    if (dist) CU(cudaMemcpyAsync(dist + q0 * k, odist.p, static_cast<size_t>(nb) * k * 8, cudaMemcpyDeviceToHost, st.s));
+  }
+  CU(cudaStreamSynchronize(st.s));
+  return 0;
+}
+
+int jb_knn_average(const long long* idx, const double* weights, long long nq, int k, const double* values, long long nr, long long w,
+                   long long ldv, long long batch_bytes, int device, double* out) {
+  if (!idx || !values || !out) return fail("null argument");
+  if (nq <= 0 || nr <= 0 || w <= 0 || ldv < w) return fail("bad shape: %lld query rows, %lld reference rows, %lld columns, pitch %lld", nq, nr, w, ldv);
+  if (nq > INT_MAX) return fail("%lld query rows: jb_knn_average takes fewer than 2^31", nq);
+  if (k < 1 || k > jb::KN_MAXK) return fail("k = %d neighbours: 1 <= k <= %d", k, jb::KN_MAXK);
+  for (long long e = 0; e < nq * k; ++e)
+    if (idx[e] < 0 || idx[e] >= nr) return fail("neighbour index %lld of query row %lld out of range [0, %lld)", idx[e], e / k, nr);
+  CU(cudaSetDevice(device));
+  // device bytes: the lists and weights (resident), and per column of a slab the reference values and the output
+  const double fixed = (weights ? 16.0 : 8.0) * static_cast<double>(nq) * k;
+  const double col_b = 8.0 * static_cast<double>(nr + nq);
+  const double avail = knn_avail();
+  if (fixed + col_b > avail)
+    return fail("kNN average needs %.2f GB of device memory for one column of %lld reference and %lld query rows; %.2f GB free",
+                (fixed + col_b) / 1e9, nr, nq, (avail > 0 ? avail : 0) / 1e9);
+  const double budget = static_cast<double>(batch_bytes) < avail - fixed ? static_cast<double>(batch_bytes) : avail - fixed;
+  long long ws = static_cast<long long>(budget / col_b);
+  if (ws < 1) ws = 1;
+  if (ws > w) ws = w;
+  if (ws > 65535LL * jb::KA_THREADS) ws = 65535LL * jb::KA_THREADS;   // column blocks in grid.y
+
+  DevArr<long long> didx;
+  DevArr<double> dw, vs, os;
+  if (didx.alloc(static_cast<size_t>(nq) * k) || (weights && dw.alloc(static_cast<size_t>(nq) * k)) || vs.alloc(static_cast<size_t>(nr) * ws) ||
+      os.alloc(static_cast<size_t>(nq) * ws)) return 1;
+  KnnStream st;   // declared after the buffers: its destructor synchronises before they are freed
+  if (st.create()) return 1;
+  CU(cudaMemcpyAsync(didx.p, idx, static_cast<size_t>(nq) * k * 8, cudaMemcpyHostToDevice, st.s));
+  if (weights) CU(cudaMemcpyAsync(dw.p, weights, static_cast<size_t>(nq) * k * 8, cudaMemcpyHostToDevice, st.s));
+  for (long long c0 = 0; c0 < w; c0 += ws) {
+    const long long wb = w - c0 < ws ? w - c0 : ws;
+    CU(cudaMemcpy2DAsync(vs.p, static_cast<size_t>(wb) * 8, values + c0, static_cast<size_t>(ldv) * 8, static_cast<size_t>(wb) * 8,
+                         static_cast<size_t>(nr), cudaMemcpyHostToDevice, st.s));
+    jb::k_knn_average<<<dim3(static_cast<unsigned>(nq), static_cast<unsigned>((wb + jb::KA_THREADS - 1) / jb::KA_THREADS)), jb::KA_THREADS, 0,
+                        st.s>>>(didx.p, weights ? dw.p : nullptr, k, vs.p, static_cast<int>(wb), os.p);
+    CU(cudaGetLastError());
+    CU(cudaMemcpy2DAsync(out + c0, static_cast<size_t>(w) * 8, os.p, static_cast<size_t>(wb) * 8, static_cast<size_t>(wb) * 8,
+                         static_cast<size_t>(nq), cudaMemcpyDeviceToHost, st.s));
+  }
   CU(cudaStreamSynchronize(st.s));
   return 0;
 }

@@ -2,7 +2,8 @@
 same default k, same printed lines), computed on the GPU (SURVEY.md 8 row N4): the O(n^2 L) distance work of FOSCTTM and
 of the kNN label transfer, and the per-feature correlation and AUROC of an imputed matrix, run as CUDA kernels behind the
 C ABI (``jb_metric_foscttm``, ``jb_metric_knn_vote``, ``jb_metric_feature_pearson``: csrc/metrics.cuh;
-``jb_metric_feature_auroc``: csrc/auroc.cuh).
+``jb_metric_feature_auroc``: csrc/auroc.cuh), and the exact kNN search and kNN regression that serve as the imputation
+baseline (``jb_knn``, ``jb_knn_average``: csrc/knn.cuh).
 
 Reference: FOSCTTM ``test_closer`` jamie/evaluation.py:65-85 (class method jamie/jamie.py:892-913), label-transfer
 accuracy ``test_LabelTA`` jamie/evaluation.py:114-132 (class method jamie/jamie.py:943-961: k = None default), per-feature
@@ -194,3 +195,114 @@ def imputation_auroc(imputed, measured, threshold=0.0, device=None):
     # 2U and 2PN are exact integers; Python's int division rounds their quotient correctly
     return np.array([u / (2 * q * (n - q)) if 0 < q < n else np.nan for u, q in zip(u2.tolist(), n_pos.tolist())],
                     np.float64)
+
+
+# Upper bound of the device working set of one query batch of kneighbors / knn_impute (the reference rows aside) and of
+# one column slab of knn_impute's average, in bytes; a sparse ``values`` is densified on the host one such slab at a time.
+KNN_BATCH_BYTES = 1 << 30
+KNN_MAX_K = 1024   # the largest k of the device search (csrc/knn.cuh KN_MAXK)
+
+
+class DeviceKnn:
+    """The two device calls of kneighbors / knn_impute (host tests substitute a numpy stand-in with the same methods)."""
+
+    @staticmethod
+    def search(query, reference, k, batch_bytes, device):
+        """jb_knn: (dist float64 [nq, k], idx int64 [nq, k]) of fp32 C-contiguous rows."""
+        nq, nr = query.shape[0], reference.shape[0]
+        idx = np.empty((nq, k), np.int64)
+        dist = np.empty((nq, k), np.float64)
+        p = lambda a: a.ctypes.data_as(C.c_void_p)   # noqa: E731
+        _lib.check(_lib.load().jb_knn(p(query), nq, p(reference), nr, query.shape[1], int(k), int(batch_bytes),
+                                      _device(device), p(idx), p(dist)))
+        return dist, idx
+
+    @staticmethod
+    def average(idx, weights, values, batch_bytes, device):
+        """jb_knn_average: float64 [nq, w] for float64 ``values`` [nr, w] with unit column stride."""
+        nq, k = idx.shape
+        out = np.empty((nq, values.shape[1]), np.float64)
+        p = lambda a: None if a is None else a.ctypes.data_as(C.c_void_p)   # noqa: E731
+        _lib.check(_lib.load().jb_knn_average(p(idx), p(weights), nq, int(k), p(values), values.shape[0], values.shape[1],
+                                              values.strides[0] // 8, int(batch_bytes), _device(device), p(out)))
+        return out
+
+
+def _knn_rows(query, reference, k):
+    """The query and reference rows as C-contiguous float32, checked; raises ValueError."""
+    q, r = np.asarray(query), np.asarray(reference)
+    if q.ndim != 2 or r.ndim != 2 or q.shape[1] != r.shape[1]:
+        raise ValueError(f'query and reference must be [n, L] matrices of one width, got {q.shape} and {r.shape}')
+    if q.shape[0] == 0 or r.shape[0] == 0 or q.shape[1] == 0:
+        raise ValueError(f'query and reference need rows and columns, got {q.shape} and {r.shape}')
+    if isinstance(k, bool) or not isinstance(k, (int, np.integer)):
+        raise ValueError(f'k must be an integer, not {k!r}')
+    if k < 1 or k > r.shape[0]:
+        raise ValueError(f'k = {k} neighbours of {r.shape[0]} reference rows: 1 <= k <= {r.shape[0]}')
+    if k > KNN_MAX_K:
+        raise ValueError(f'k = {k}: the device search takes at most {KNN_MAX_K} neighbours')
+    with np.errstate(over='ignore'):
+        q32, r32 = _f32(q), _f32(r)
+    for name, a in (('query', q32), ('reference', r32)):
+        if not np.isfinite(a).all():
+            raise ValueError(f'{name} has non-finite values (after rounding to float32)')
+    return q32, r32
+
+
+def kneighbors(query, reference, k, device=None, backend=DeviceKnn):
+    """The k nearest reference rows of every query row in euclidean distance, searched exactly on the GPU (``jb_knn``):
+    (dist float64 [nq, k], idx int64 [nq, k]), each row in ascending distance, equal distances by the lowest reference
+    index. The same as ``NearestNeighbors(n_neighbors=k, algorithm='brute').fit(reference).kneighbors(query)`` on data
+    without exact ties. Rows are rounded to float32, as ``test_closer`` and ``test_LabelTA`` do; distances are float64
+    sums of squared differences, so they carry no cancellation. 1 <= k <= min(1024, nr)."""
+    q32, r32 = _knn_rows(query, reference, k)
+    return backend.search(q32, r32, int(k), KNN_BATCH_BYTES, device)
+
+
+def knn_weights(dist, weights):
+    """sklearn's neighbour weights: None for 'uniform'; for 'distance' 1 / d, except that a row with a zero distance
+    weighs its zero-distance neighbours 1 and the others 0."""
+    if weights == 'uniform':
+        return None
+    with np.errstate(divide='ignore'):
+        w = 1.0 / dist
+    inf = np.isinf(w)
+    rows = inf.any(axis=1)
+    w[rows] = inf[rows]
+    return np.ascontiguousarray(w, np.float64)
+
+
+def knn_impute(query, reference, values, k=5, weights='uniform', device=None, backend=DeviceKnn):
+    """kNN regression on the GPU: for every query row the average of ``values`` over its k nearest ``reference`` rows
+    (``kneighbors``), uniform or weighted by inverse distance (``weights='distance'``, sklearn's rules), float64 [nq, d].
+    The same as ``KNeighborsRegressor(n_neighbors=k, weights=weights, algorithm='brute').fit(reference, values)
+    .predict(query)``. ``values`` [nr, d] is a dense array (read as float64) or any scipy.sparse matrix; either goes to the
+    device in column slabs, and a sparse one is densified one slab at a time."""
+    if weights not in ('uniform', 'distance'):
+        raise ValueError(f"weights must be 'uniform' or 'distance', not {weights!r}")
+    q32, r32 = _knn_rows(query, reference, k)
+    (nq, _), (nr, _) = q32.shape, r32.shape
+    V = values if _is_sparse(values) else np.asarray(values, np.float64)
+    if V.ndim != 2 or V.shape[0] != nr:
+        raise ValueError(f'values must be [{nr}, d] (one row per reference row), got shape {V.shape}')
+    d = V.shape[1]
+    if _is_sparse(V):
+        V = V.tocsc(copy=True)
+        V.sum_duplicates()
+        finite = np.isfinite(V.data).all()
+    else:
+        finite = np.isfinite(V).all()
+    if not finite:
+        raise ValueError('values has non-finite values')
+    dist, idx = backend.search(q32, r32, int(k), KNN_BATCH_BYTES, device)
+    w = knn_weights(dist, weights)
+    if d == 0:
+        return np.zeros((nq, 0), np.float64)
+    if not _is_sparse(V):
+        return backend.average(idx, w, np.ascontiguousarray(V), KNN_BATCH_BYTES, device)
+    out = np.empty((nq, d), np.float64)
+    cw = max(1, KNN_BATCH_BYTES // (8 * (nr + nq)))
+    for c0 in range(0, d, cw):
+        out[:, c0:c0 + cw] = backend.average(idx, w, np.ascontiguousarray(V[:, c0:c0 + cw].toarray(), np.float64),
+                                             KNN_BATCH_BYTES, device)
+    return out

@@ -700,6 +700,17 @@ class JAMIE(UnionCom):
         return shap_values(self, data, modality, background, outputs=outputs, space=space, n_permutations=n_permutations,
                            seed=seed)
 
+    def knn_predict(self, data, modality, reference, k=5, weights='uniform'):
+        """Impute the other modality of ``data`` (raw rows of modality ``modality``) by nearest neighbours in the joint
+        embedding: each row's imputation averages the measured raw rows of ``reference`` (the other modality, dense or
+        scipy.sparse where ``transform_one`` takes it) over its k nearest reference rows, uniformly or by inverse distance
+        (``weights='distance'``). The baseline that ``modal_predict``'s decoder imputation is judged against; float64
+        [n, d_other_raw]. Exact search and averaging on the GPU (``evaluation.knn_impute``)."""
+        from .evaluation import knn_impute
+        other = (modality + 1) % self.dataset_num
+        return knn_impute(self.transform_one(data, modality), self.transform_one(reference, other), reference, k=k,
+                          weights=weights, device=self._cuda_index())
+
     # ------------------------------------------------------------------------------------------------ metrics
     def test_closer(self, integrated_data, distance_metric=None):
         """Test fraction of samples closer than the true match (jamie/jamie.py:892-913; prints ``foscttm: ...``)"""
