@@ -290,6 +290,19 @@ int jb_knn(const float* query, long long nq, const float* ref, long long nr, int
 int jb_knn_average(const long long* idx, const double* weights, long long nq, int k, const double* values, long long nr,
                    long long w, long long ldv, long long batch_bytes, int device, double* out);
 
+/* Silhouette sums on the GPU (csrc/silhouette.cuh; no engine handle; host pointers in, synchronous). They replace the
+ * O(n^2 L) pair loop of sklearn's silhouette_samples on the host.
+ *   x [n, L] row-major fp32, sorted by label: label c holds rows [label_off[c], label_off[c + 1]) (int64 label_off
+ *   [n_labels + 1], 0 first, n last, every label non-empty; 2 <= n_labels <= n; n < 2^31). With d(i, j) the sqrt of the
+ *   float64 sum of squared fp32 differences (the tile arithmetic of jb_metric_foscttm) and S[i, c] = sum over the rows
+ *   j of label c of d(i, j):  intra[i] = S[i, l_i],  inter[i] = min over c != l_i of S[i, c] / n_c  (float64 [n], the two
+ *   arrays of sklearn's _silhouette_reduce before the intra division). The rows stay on the device and the query rows go
+ *   in batches whose workspace fits in batch_bytes. No floating-point atomics: results do not depend on batch_bytes or
+ *   the device. Refuses, before any allocation, a problem whose rows and one query row's workspace do not fit in free
+ *   device memory. */
+int jb_silhouette(const float* x, long long n, int L, const long long* label_off, int n_labels, long long batch_bytes,
+                  int device, double* intra, double* inter);
+
 /* Distances of the F estimation (compute_distances, jamie/jamie.py:839-890; the default distance_mode 'geodesic' is
  * unioncom.utils.geodesic_distances of unioncom==0.4.0, restated and unpinned in jamie_b200/correspondence.py).
  * A jb_dist handle owns one n x n float64 matrix D on one device and a stream; host pointers throughout.

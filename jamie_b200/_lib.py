@@ -71,6 +71,7 @@ SIGNATURES = {
     'jb_metric_feature_auroc': (C.c_int, [_P, _LL, _LL, _P, _P, _LL, C.c_int, _P, _P]),
     'jb_knn': (C.c_int, [_P, _LL, _P, _LL, C.c_int, C.c_int, _LL, C.c_int, _P, _P]),
     'jb_knn_average': (C.c_int, [_P, _P, _LL, C.c_int, _P, _LL, _LL, _LL, _LL, C.c_int, _P]),
+    'jb_silhouette': (C.c_int, [_P, _LL, C.c_int, _P, C.c_int, _LL, C.c_int, _P, _P]),
     'jb_dist_create': (C.c_int, [_LL, C.c_int, C.POINTER(_P)]),
     'jb_dist_destroy': (None, [_P]),
     'jb_dist_accumulate': (C.c_int, [_P, C.c_int, _P, _LL, _LL]),

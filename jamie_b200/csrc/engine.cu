@@ -39,6 +39,7 @@
 #include "shapley.cuh"
 #include "auroc.cuh"
 #include "knn.cuh"
+#include "silhouette.cuh"
 
 namespace {
 
@@ -2232,6 +2233,73 @@ int jb_knn_average(const long long* idx, const double* weights, long long nq, in
     CU(cudaGetLastError());
     CU(cudaMemcpy2DAsync(out + c0, static_cast<size_t>(w) * 8, os.p, static_cast<size_t>(wb) * 8, static_cast<size_t>(wb) * 8,
                          static_cast<size_t>(nq), cudaMemcpyDeviceToHost, st.s));
+  }
+  CU(cudaStreamSynchronize(st.s));
+  return 0;
+}
+
+// ---------------------------------------------------------------------------------------------- silhouette sums
+
+int jb_silhouette(const float* x, long long n, int L, const long long* label_off, int n_labels, long long batch_bytes,
+                  int device, double* intra, double* inter) {
+  if (!x || !label_off || !intra || !inter) return fail("null argument");
+  if (n <= 0 || L <= 0) return fail("bad embedding shape: %lld rows, %d columns", n, L);
+  if (n > INT_MAX) return fail("%lld rows: jb_silhouette takes fewer than 2^31", n);
+  if (n_labels < 2 || n_labels > n) return fail("%d labels of %lld rows: 2 <= labels <= rows", n_labels, n);
+  if (label_off[0] != 0 || label_off[n_labels] != n)
+    return fail("label offsets must run from 0 to %lld rows, got %lld to %lld", n, label_off[0], label_off[n_labels]);
+  for (int c = 0; c < n_labels; ++c)
+    if (label_off[c + 1] <= label_off[c]) return fail("label %d is empty or its offsets decrease (%lld, %lld)", c, label_off[c], label_off[c + 1]);
+  // per chunk of reference rows: its first label and the offset of its slots (one per label it holds)
+  const long long nch = (n + jb::SL_CHUNK - 1) / jb::SL_CHUNK;
+  std::vector<long long> slot_base(nch + 1, 0);
+  std::vector<int> first_label(nch);
+  for (long long ch = 0, c = 0; ch < nch; ++ch) {
+    const long long r0 = ch * jb::SL_CHUNK, r1 = (r0 + jb::SL_CHUNK < n ? r0 + jb::SL_CHUNK : n) - 1;
+    while (label_off[c + 1] <= r0) ++c;
+    long long c2 = c;
+    while (label_off[c2 + 1] <= r1) ++c2;
+    first_label[ch] = static_cast<int>(c);
+    slot_base[ch + 1] = slot_base[ch] + (c2 - c + 1);
+  }
+  const long long P = slot_base[nch];
+  CU(cudaSetDevice(device));
+  // device bytes: the rows and the label / slot tables (resident), and per query row of a batch its P slots and outputs
+  const double res_b = 4.0 * static_cast<double>(n) * L + 8.0 * (n_labels + 1) + 12.0 * static_cast<double>(nch) + 8.0;
+  const double row_b = 8.0 * static_cast<double>(P) + 16.0;
+  const double avail = knn_avail();
+  if (res_b + row_b > avail)
+    return fail("silhouette needs %.2f GB of device memory for %lld rows and one query row's workspace; %.2f GB free",
+                (res_b + row_b) / 1e9, n, (avail > 0 ? avail : 0) / 1e9);
+  const double budget = static_cast<double>(batch_bytes) < avail - res_b ? static_cast<double>(batch_bytes) : avail - res_b;
+  long long nqb = static_cast<long long>(budget / row_b);
+  if (nqb > n) nqb = n;
+  if (nqb > 65535LL * jb::MT_TILE) nqb = 65535LL * jb::MT_TILE;   // query tiles in grid.y
+  if (nqb >= jb::MT_TILE) nqb -= nqb % jb::MT_TILE;
+  if (nqb < 1) nqb = 1;
+  CU(cudaFuncSetAttribute(jb::k_sil_partial, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(jb::SL_SMEM)));
+
+  DevArr<float> dx;
+  DevArr<long long> doff, dbase;
+  DevArr<int> dfirst;
+  DevArr<double> ws, da, db;
+  if (dx.alloc(static_cast<size_t>(n) * L) || doff.alloc(n_labels + 1) || dbase.alloc(nch + 1) || dfirst.alloc(nch) ||
+      ws.alloc(static_cast<size_t>(nqb) * P) || da.alloc(nqb) || db.alloc(nqb)) return 1;
+  KnnStream st;   // declared after the buffers: its destructor synchronises before they are freed
+  if (st.create()) return 1;
+  CU(cudaMemcpyAsync(dx.p, x, static_cast<size_t>(n) * L * 4, cudaMemcpyHostToDevice, st.s));
+  CU(cudaMemcpyAsync(doff.p, label_off, static_cast<size_t>(n_labels + 1) * 8, cudaMemcpyHostToDevice, st.s));
+  CU(cudaMemcpyAsync(dbase.p, slot_base.data(), static_cast<size_t>(nch + 1) * 8, cudaMemcpyHostToDevice, st.s));
+  CU(cudaMemcpyAsync(dfirst.p, first_label.data(), static_cast<size_t>(nch) * 4, cudaMemcpyHostToDevice, st.s));
+  for (long long q0 = 0; q0 < n; q0 += nqb) {
+    const long long nb = n - q0 < nqb ? n - q0 : nqb;
+    jb::k_sil_partial<<<dim3(static_cast<unsigned>(nch), static_cast<unsigned>((nb + jb::MT_TILE - 1) / jb::MT_TILE)), jb::MT_THREADS,
+                        jb::SL_SMEM, st.s>>>(dx.p, n, L, q0, nb, doff.p, dbase.p, dfirst.p, ws.p);
+    jb::k_sil_finish<<<static_cast<unsigned>((nb + jb::SF_THREADS - 1) / jb::SF_THREADS), jb::SF_THREADS, 0, st.s>>>(
+        ws.p, q0, nb, doff.p, n_labels, dbase.p, dfirst.p, da.p, db.p);
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(intra + q0, da.p, static_cast<size_t>(nb) * 8, cudaMemcpyDeviceToHost, st.s));
+    CU(cudaMemcpyAsync(inter + q0, db.p, static_cast<size_t>(nb) * 8, cudaMemcpyDeviceToHost, st.s));
   }
   CU(cudaStreamSynchronize(st.s));
   return 0;

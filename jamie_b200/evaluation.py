@@ -2,8 +2,10 @@
 same default k, same printed lines), computed on the GPU (SURVEY.md 8 row N4): the O(n^2 L) distance work of FOSCTTM and
 of the kNN label transfer, and the per-feature correlation and AUROC of an imputed matrix, run as CUDA kernels behind the
 C ABI (``jb_metric_foscttm``, ``jb_metric_knn_vote``, ``jb_metric_feature_pearson``: csrc/metrics.cuh;
-``jb_metric_feature_auroc``: csrc/auroc.cuh), and the exact kNN search and kNN regression that serve as the imputation
-baseline (``jb_knn``, ``jb_knn_average``: csrc/knn.cuh).
+``jb_metric_feature_auroc``: csrc/auroc.cuh), the exact kNN search and kNN regression that serve as the imputation
+baseline (``jb_knn``, ``jb_knn_average``: csrc/knn.cuh), and the silhouette coefficients of an embedding under a labelling
+(``jb_silhouette``: csrc/silhouette.cuh; sklearn's ``silhouette_samples`` / ``silhouette_score``), scored with cell types
+for how well they separate and with the modality for how well the modalities mix.
 
 Reference: FOSCTTM ``test_closer`` jamie/evaluation.py:65-85 (class method jamie/jamie.py:892-913), label-transfer
 accuracy ``test_LabelTA`` jamie/evaluation.py:114-132 (class method jamie/jamie.py:943-961: k = None default), per-feature
@@ -306,3 +308,98 @@ def knn_impute(query, reference, values, k=5, weights='uniform', device=None, ba
         out[:, c0:c0 + cw] = backend.average(idx, w, np.ascontiguousarray(V[:, c0:c0 + cw].toarray(), np.float64),
                                              KNN_BATCH_BYTES, device)
     return out
+
+
+# Upper bound of the device working set of one query batch of silhouette_samples (the rows aside), in bytes.
+SILHOUETTE_BATCH_BYTES = 1 << 30
+
+
+class DeviceSilhouette:
+    """The device call of silhouette_samples (host tests substitute a numpy stand-in with the same method)."""
+
+    @staticmethod
+    def sums(x_sorted, label_off, batch_bytes, device):
+        """jb_silhouette: (intra, inter) float64 [n] of fp32 C-contiguous rows sorted by label, label c holding rows
+        label_off[c] .. label_off[c + 1]: the sum of the distances to the row's own label, and the least mean distance to
+        another label."""
+        n, L = x_sorted.shape
+        off = np.ascontiguousarray(label_off, np.int64)
+        intra, inter = np.empty(n, np.float64), np.empty(n, np.float64)
+        p = lambda a: a.ctypes.data_as(C.c_void_p)   # noqa: E731
+        _lib.check(_lib.load().jb_silhouette(p(x_sorted), n, L, p(off), len(off) - 1, int(batch_bytes), _device(device),
+                                             p(intra), p(inter)))
+        return intra, inter
+
+
+def silhouette_samples(X, labels, metric='euclidean', device=None, backend=DeviceSilhouette):
+    """The silhouette coefficient of every row, float64 [n]: the same as ``sklearn.metrics.silhouette_samples(X, labels)``
+    with its O(n^2 L) pair work on the GPU (``jb_silhouette``). With a the mean distance of row i to the other rows of its
+    label and b the least mean distance to the rows of another label, s = (b - a) / max(a, b); a row alone in its label,
+    and a row with a = b = 0, gives 0. Rows are rounded to float32, as ``test_closer`` and ``kneighbors`` do; distances
+    are the sqrt of float64 sums of squared differences, so they carry no cancellation. Scored with cell types as labels
+    it measures how well types separate in a joint embedding; with the modality (0 / 1), how well the modalities mix."""
+    if metric != 'euclidean':
+        raise ValueError(f"metric must be 'euclidean', the only one supported, not {metric!r}")
+    if _is_sparse(X):
+        raise ValueError('X must be a dense array')
+    x, lab = np.asarray(X), np.asarray(labels)
+    if x.ndim != 2:
+        raise ValueError(f'X must be an [n, L] matrix, got shape {x.shape}')
+    if lab.ndim != 1 or lab.shape[0] != x.shape[0]:
+        raise ValueError(f'labels must be one label per row of X ({x.shape[0]}), got shape {lab.shape}')
+    n = x.shape[0]
+    if n == 0 or x.shape[1] == 0:
+        raise ValueError(f'X needs rows and columns, got shape {x.shape}')
+    if n >= 1 << 31:
+        raise ValueError(f'{n} rows: silhouette_samples takes fewer than 2^31')
+    with np.errstate(over='ignore'):
+        x32 = _f32(x)
+    if not np.isfinite(x32).all():
+        raise ValueError('X has non-finite values (after rounding to float32)')
+    classes, codes = np.unique(lab, return_inverse=True)   # sklearn's LabelEncoder
+    codes = codes.ravel()
+    if not 1 < len(classes) < n:
+        raise ValueError('Number of labels is %d. Valid values are 2 to n_samples - 1 (inclusive)' % len(classes))
+    freq = np.bincount(codes)
+    order = np.argsort(codes, kind='stable')
+    label_off = np.concatenate([[0], np.cumsum(freq)]).astype(np.int64)
+    intra_s, inter_s = backend.sums(np.ascontiguousarray(x32[order]), label_off, SILHOUETTE_BATCH_BYTES, device)
+    intra, inter = np.empty(n, np.float64), np.empty(n, np.float64)
+    intra[order], inter[order] = intra_s, inter_s
+    # sklearn's own finish, in its order
+    denom = (freq - 1).take(codes, mode='clip')
+    with np.errstate(divide='ignore', invalid='ignore'):
+        intra /= denom
+    sil = inter - intra
+    with np.errstate(divide='ignore', invalid='ignore'):
+        sil /= np.maximum(intra, inter)
+    return np.nan_to_num(sil)
+
+
+def silhouette_score(X, labels, metric='euclidean', sample_size=None, random_state=None, device=None,
+                     backend=DeviceSilhouette):
+    """The mean silhouette coefficient, ``float(np.mean(silhouette_samples(X, labels)))``: the same as
+    ``sklearn.metrics.silhouette_score``. With ``sample_size``, it scores the rows
+    ``check_random_state(random_state).permutation(n)[:sample_size]``, as sklearn draws them."""
+    if sample_size is not None:
+        if isinstance(sample_size, bool) or not isinstance(sample_size, (int, np.integer)) or sample_size < 1:
+            raise ValueError(f'sample_size must be a positive integer or None, not {sample_size!r}')
+        if _is_sparse(X):
+            raise ValueError('X must be a dense array')
+        x, lab = np.asarray(X), np.asarray(labels)
+        if x.ndim != 2 or lab.ndim != 1 or lab.shape[0] != x.shape[0]:
+            raise ValueError(f'X must be an [n, L] matrix with one label per row, got shapes {x.shape} and {lab.shape}')
+        idx = _random_state(random_state).permutation(x.shape[0])[:sample_size]
+        X, labels = x[idx], lab[idx]
+    return float(np.mean(silhouette_samples(X, labels, metric=metric, device=device, backend=backend)))
+
+
+def _random_state(seed):
+    """sklearn's check_random_state: numpy's global RandomState for None, a new one for an integer, or the instance."""
+    if seed is None or seed is np.random:
+        return np.random.mtrand._rand
+    if isinstance(seed, (int, np.integer)) and not isinstance(seed, bool):
+        return np.random.RandomState(seed)
+    if isinstance(seed, np.random.RandomState):
+        return seed
+    raise ValueError(f'{seed!r} cannot be used to seed a numpy.random.RandomState instance')
